@@ -2,7 +2,7 @@
 """Benchmark of the VoiceFixer inference hot path (BASELINE.json metric: clips/sec on 44.1 kHz 10 s clips).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--workload gsr|ssr|longform] [--batch B] [--seconds S] [--minutes M]
+                    [--workload gsr|ssr|longform] [--batch B] [--seconds S] [--minutes M] [--dump-outputs DIR]
 
 Default workload `gsr` (what the driver runs): a step = one pass of the whole hot path (STFT+mel -> ResUNet ->
 vocoder -> peak-normalise -> trim) over one batch of B synthetic clips per GPU (configs[1] of BASELINE.json: batch
@@ -16,6 +16,8 @@ host-buffer entry point (pinned host buffers, H2D + D2H inside the timed region)
 golden clip riding in row 0 of the benchmarked batch; `cpu_baseline` = the oracle timed on host cores.
 `--impl reference` times the reference algorithm on the host CPU (the oracle port - the reference itself is a Python
 tree that cannot travel to the GPU box) on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the timed path returned in its last timed step as DIR/<name>.npy (float32, rank 0):
+inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -34,7 +36,8 @@ SR, HOP = 44100, 441
 METRIC = "clips_per_sec_10s_44k1"
 UNET_GFLOP_PER_CLIP_T1024 = 190.16          # SURVEY.md 8(d): mel UNet, T' = 1024
 SSR_GFLOP_PER_CLIP_T1024 = 1597.95          # SURVEY.md 8(d): unet_v2, T' = 1024
-REF_STEP_BUDGET_S = 150.0                   # --impl reference: bound on timed CPU work (the whole run must end in minutes)
+REF_STEP_BUDGET_S = 150.0                   # --impl reference: bound on CPU warm-up work (the whole run must end in minutes)
+DUMP_BUDGET_BYTES = 64 * 10**6              # --dump-outputs: all files together
 
 
 def load_peaks():
@@ -94,6 +97,20 @@ def synth_batch(batch, n, seed):
     return sig / sig.abs().amax(dim=1, keepdim=True) * (0.3 + 0.7 * torch.rand(batch, 1, generator=g))
 
 
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy in float32.  One larger than its share of DUMP_BUDGET_BYTES is replaced
+    by a fixed sample: every step-th element of the flattened array from a seeded offset, the same on every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    keep = (DUMP_BUDGET_BYTES // len(arrays) - 128) // 4         # 128 = .npy header
+    for name, t in arrays.items():
+        a = t.detach().to("cpu", torch.float32).numpy()
+        if a.size > keep:
+            step = -(-a.size // keep)
+            a = a.reshape(-1)[int(np.random.default_rng(0).integers(step))::step]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def load_golden(name):
     import numpy as np
     p = os.path.join(ROOT, "tests", "golden", name)
@@ -119,7 +136,7 @@ def best_cpu_threads(fn, candidates):
 def cpu_reference(workload, seconds, steps, warmup, threads=None):
     """The reference algorithm (oracle port, pinned against the reference's own modules where they import) on the host
     CPU, one clip per step as the reference runs it (batch 1, eval_gsr_voicefixer.py:19-21), warm-up on the FULL clip.
-    Returns (clips/s, s/step, threads, steps actually timed, note)."""
+    Returns (clips/s, s/step, threads, note, output of the last timed step)."""
     from oracle import vf_oracle as O
     from voicefixer_main_b200.weights import make_ssr_state, make_state
     n = int(seconds * SR)
@@ -146,17 +163,10 @@ def cpu_reference(workload, seconds, steps, warmup, threads=None):
                 break
             step(wav)
         t0 = time.perf_counter()
-        step(wav)
-        one = time.perf_counter() - t0
-        k = max(1, min(steps, int(REF_STEP_BUDGET_S / max(one, 1e-3))))
-        if k < steps:
-            note = (note + "; " if note else "") + f"timed steps capped at {k} of {steps}: one step takes {one:.1f} s and the run is bounded to ~{REF_STEP_BUDGET_S:.0f} s of CPU work"
-        dt = one
-        t0 = time.perf_counter()
-        for _ in range(k - 1):
-            step(wav)
-        dt += time.perf_counter() - t0
-    return k / dt, dt / k, threads, k, note
+        for _ in range(steps):
+            out = step(wav)
+        dt = time.perf_counter() - t0
+    return steps / dt, dt / steps, threads, note, out
 
 
 def run_reference(args):
@@ -165,7 +175,10 @@ def run_reference(args):
         return
     seconds = args.seconds if args.seconds else (3.0 if args.workload == "ssr" else 10.0)
     wl = "ssr" if args.workload == "ssr" else "gsr"
-    cps, spc, threads, k, note = cpu_reference(wl, seconds, max(1, args.steps), max(1, args.warmup))
+    cps, spc, threads, note, out = cpu_reference(wl, seconds, args.steps, max(1, args.warmup))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"restored": out})
+    k = args.steps
     what = ("ssr_unet (unet_v2 + ISTFT) forward" if wl == "ssr" else "gsr_voicefixer handler path")
     line = {
         "impl": "reference", "metric": METRIC if wl == "gsr" and seconds == 10.0 else f"clips_per_sec_{seconds:g}s_44k1", "value": cps, "unit": "clips/s",
@@ -355,6 +368,7 @@ def run_b200(args):
     l0 = eng.launch_count()
     ms = timed_loop(step_dev, args.steps, barrier, dev, vdist)
     launches = eng.launch_count() - l0
+    restored = dev_out.cpu() if args.dump_outputs and rank == 0 else None      # before the profiling steps rewrite it
     # ---- end to end through the public host API (pinned host in/out, copies inside the timed region)
     for _ in range(min(2, args.warmup)):
         step_host()
@@ -365,6 +379,8 @@ def run_b200(args):
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"restored": restored})
     parity = None
     if gold is not None:
         _, log_mel = eng.restore_stages(B, n)
@@ -394,7 +410,8 @@ def run_b200(args):
     e2e = clips * args.steps / (ms_e2e * 1e-3)
     cpu = None
     if not args.no_cpu_baseline:
-        cps, spc, threads, k, note = cpu_reference("ssr" if ssr else "gsr", seconds, 2, 1)
+        k = 2
+        cps, spc, threads, note, _ = cpu_reference("ssr" if ssr else "gsr", seconds, k, 1)
         cpu = {"value": cps, "unit": "clips/s", "cores": threads, "kind": "port",
                "sample": f"{k} x one {seconds:g} s clip (batch 1), oracle port of the reference, torch CPU fp32, best thread count {threads} of {os.cpu_count()} host cores",
                "rtf": cps * seconds}
@@ -486,13 +503,16 @@ def run_longform(args):
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    out_m = restore_longform(model, dev_in, max_batch=gb)
+    for _ in range(args.steps):
+        out_m = restore_longform(model, dev_in, max_batch=gb)
     e1.record()
     torch.cuda.synchronize()
-    ms_m = e0.elapsed_time(e1)
+    ms_m = e0.elapsed_time(e1) / args.steps
     res["margins_30s_windows_2s_context"] = {"ms_per_stream": ms_m, "rtf": n / SR / (ms_m * 1e-3), "windows": (n + 30 * SR - 1) // (30 * SR)}
     sampler.stop_flag = True
     eng.check_errors()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"handler_hard_cuts": ref_out, f"segments_batched_{gb}": out_host, "margins": out_m})
     # parity of one 60 s segment against the oracle (the reference's handler on the CPU)
     parity = None
     if not args.no_cpu_baseline:
@@ -530,7 +550,11 @@ def main():
     ap.add_argument("--no-graphs", action="store_true", help="launch every kernel individually instead of replaying CUDA graphs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-out", default="", help="write the per-launch profile (JSON) to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

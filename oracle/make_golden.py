@@ -1,6 +1,7 @@
 """Generate tests/golden/*.npz from the REFERENCE ITSELF.  TEST INFRASTRUCTURE ONLY.
 
-Run in the build container (needs /root/reference):  python oracle/make_golden.py
+Needs the reference tree at ref_import.REFERENCE_ROOT:
+    python oracle/make_golden.py [ssr | small | reference | longform]
 
 Every output below is produced by the reference's own modules imported unmodified
 (oracle/ref_import.py): FDomainHelper + MelScale (stage A), VoiceFixer.forward ->
@@ -102,10 +103,124 @@ def main_small():
     print("stage_b_small_t101 written")
 
 
+STRIDE = 7       # reference outputs are stored as out.reshape(-1)[::STRIDE]: 7 is coprime to the 128 mel bins and the hop
+
+
+def sample(t: torch.Tensor, stride: int = STRIDE) -> np.ndarray:
+    return t.detach().reshape(-1)[::stride].contiguous().numpy()
+
+
+def main_reference():
+    """What tests/test_oracle_vs_reference.py and test_host_cpu.py::test_arch_keys_match_reference_state_dict compare
+    the restatement with (reference_oracle.npz): the reference's own modules run on the inputs those tests build,
+    outputs stored as a strided sample, and the UNet state-dict keys and shapes in registration order."""
+    from voicefixer_main_b200.arch import UNET_PREFIX
+    torch.set_num_threads(os.cpu_count() or 1)
+    sd = make_state(SEED)
+    model, _ = ref_import.build_reference_model(sd)
+    ref_import.install_shims()
+    from tools.pytorch.pytorch_util import from_log, to_log
+    from tools.utils import trim_center
+    g = {"fingerprint": state_fingerprint(sd), "stride": np.int64(STRIDE)}
+
+    fb = model.mel.fb
+    nz = torch.nonzero(fb.reshape(-1))[:, 0]
+    g.update(fb_shape=np.array(fb.shape), fb_index=nz.int().numpy(), fb_value=fb.reshape(-1)[nz].numpy())
+
+    gl = torch.Generator().manual_seed(23)
+    x = torch.rand(3, 1, 7, 128, generator=gl) * 3
+    x[0, 0, 0, :4] = 0
+    y = torch.randn(3, 1, 7, 128, generator=gl) * 4
+    g.update(to_log=to_log(x).numpy(), from_log=from_log(y).numpy())
+    try:
+        to_log(-x - 1)
+        g["to_log_rejects_negative"] = np.bool_(False)
+    except AssertionError:
+        g["to_log_rejects_negative"] = np.bool_(True)
+
+    starts = []
+    for le, lr in ((20, 14), (443646, 441000), (16, 16)):
+        est = torch.arange(float(le))[None, None]
+        out = trim_center(est, torch.zeros(1, 1, lr))[0]
+        s = int(out[0, 0, 0])
+        assert torch.equal(out, est[..., s:s + lr])            # a contiguous window: its start says it all
+        starts.append((le, lr, s))
+    g["trim_center"] = np.array(starts, dtype=np.int64)
+
+    with torch.no_grad():
+        gm = torch.Generator().manual_seed(3)
+        for t in (64, 101, 130):
+            mel = 10 ** (torch.randn(2, 1, t, 128, generator=gm) - 1)
+            g[f"unet_t{t}"] = sample(model(mel)["mel"])
+        wav = O.synth_clips(2, 30000, seed=9)
+        g["handler"] = sample(ref_import.reference_handler_batch(model, wav, seg_samples=12000))
+
+        ssr = {k.replace(UNET_PREFIX, "generator.unet."): v for k, v in sd.items() if k.startswith(UNET_PREFIX)}
+        net = ref_import.build_reference_unet_v2(ssr)
+        for n in (63 * 441, 70 * 441 + 17):
+            w = O.synth_clips(1, n, seed=n)[:, None, :]
+            sp, _, _ = O.wav_to_spectrogram_phase(w)
+            g[f"ssr_n{n}"] = sample(net(sp, w)["wav"])
+
+        small = ref_import.build_reference_unet_small(sd)
+        mel = 10 ** (torch.randn(1, 1, 101, 128, generator=torch.Generator().manual_seed(4)) - 1)
+        g["small"] = sample(small(to_log(mel))["mel"] + to_log(mel))
+        g["small_full"] = sample(model(mel)["mel"])
+
+    keys = [(k[len(UNET_PREFIX):], tuple(v.shape)) for k, v in model.state_dict().items() if k.startswith(UNET_PREFIX)]
+    g["unet_keys"] = np.array([k for k, _ in keys])
+    g["unet_shapes"] = np.array([list(s) + [0] * (4 - len(s)) for _, s in keys], dtype=np.int32)   # zero-padded
+    g["unet_ndims"] = np.array([len(s) for _, s in keys], dtype=np.int32)
+    np.savez_compressed(os.path.join(GOLD, "reference_oracle.npz"), **g)
+    print("reference_oracle.npz written")
+
+
+def main_longform():
+    """What tests/test_longform_cpu.py compares the overlap-add mirrors with: the reference's own LambdaOverlapAdd
+    (tools/dsp/overlapadd_boxcar.py and tools/dsp/overlapadd.py, loaded unmodified) run over that test's toy network,
+    signals and cases: every second output sample (the comparison is bit for bit) and the chunk shapes that reached the
+    network."""
+    import importlib.util
+
+    def load(path, name):
+        spec = importlib.util.spec_from_file_location(name, path)
+        mod = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mod)
+        return mod
+
+    sys.path.insert(0, os.path.join(ROOT, "tests"))              # the test module imports its conftest
+    T = load(os.path.join(ROOT, "tests", "test_longform_cpu.py"), "test_longform_cpu")
+    boxcar = load(os.path.join(ref_import.REFERENCE_ROOT, "tools", "dsp", "overlapadd_boxcar.py"), "ref_overlapadd_boxcar")
+    ola = load(os.path.join(ref_import.REFERENCE_ROOT, "tools", "dsp", "overlapadd.py"), "ref_overlapadd")
+    g = {"stride": np.int64(2)}
+    for n, w, m in T.CASES:
+        for windowed in (False, True):
+            net = T.ToyNet()
+            ref = boxcar.LambdaOverlapAdd(nnet=net, n_src=1, window_size=w, in_margin=m, window="hann", reorder_chunks=False)
+            ref.use_window = windowed
+            key = T.boxcar_key(n, w, m, windowed)
+            g[key] = sample(ref(T._signal(n)), 2)
+            g[key + "_calls"] = np.array(sorted(net.calls), dtype=np.int64)
+    for n, w, hop in T.OLA_CASES:
+        for windowed in (True, False):
+            net = T.ToyNet()
+            ref = ola.LambdaOverlapAdd(nnet=net, n_src=1, window_size=w, hop_size=hop, window="hann", reorder_chunks=False)
+            ref.use_window = windowed
+            key = T.ola_key(n, w, hop, windowed)
+            g[key] = sample(ref(T._signal(n)), 2)
+            g[key + "_calls"] = np.array(net.calls, dtype=np.int64)
+    np.savez_compressed(os.path.join(GOLD, "reference_longform.npz"), **g)
+    print("reference_longform.npz written")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "ssr":
         main_ssr()
     elif len(sys.argv) > 1 and sys.argv[1] == "small":
         main_small()
+    elif len(sys.argv) > 1 and sys.argv[1] == "reference":
+        main_reference()
+    elif len(sys.argv) > 1 and sys.argv[1] == "longform":
+        main_longform()
     else:
         main()

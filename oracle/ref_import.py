@@ -1,8 +1,7 @@
 """Import the reference's own modules UNMODIFIED from /root/reference.  TEST INFRASTRUCTURE ONLY.
 
-Works only in the build container (the GPU box has no /root/reference); used by
-oracle/make_golden.py to generate tests/golden/ and by
-tests/test_oracle_vs_reference.py to pin oracle/vf_oracle.py against the real code.
+Works only where the reference tree exists; used by oracle/make_golden.py to store
+what the reference computes under tests/golden/, which the tests compare against.
 
 Third-party packages the reference imports but this image lacks are replaced by
 stubs in sys.modules *before* the import:
@@ -16,7 +15,8 @@ stubs in sys.modules *before* the import:
   empty modules (never called on the inference path we exercise).
 
 Modules that run `git.Repo("", search_parent_directories=True)` at import
-(models/components/unet.py:5) need the cwd inside a git work tree: /root/repo is one.
+(models/components/unet.py:5) need the cwd inside a git work tree: a git checkout of
+this repository is one.
 """
 import os
 import sys

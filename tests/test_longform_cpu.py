@@ -1,20 +1,19 @@
 """Long-form overlap-add with context margins (voicefixer_main_b200/longform.py) - host logic, CPU only.
 
-The mirror is checked (a) against the reference's own LambdaOverlapAdd (tools/dsp/overlapadd_boxcar.py:338-534),
-imported unmodified where /root/reference exists, with identical toy networks, and (b) through properties that
-need no reference: the batched schedule equals the sequential one, and with a margin at least as long as the
-network's receptive field the chunking is invisible."""
-import importlib.util
-import os
+The mirror is checked (a) against the reference's own LambdaOverlapAdd (tools/dsp/overlapadd_boxcar.py:338-534):
+tests/golden/reference_longform.npz holds every second sample of what that class, imported unmodified, returned for
+the toy network and signals below (python oracle/make_golden.py longform), and (b) through properties that need no
+reference: the batched schedule equals the sequential one, and with a margin at least as long as the network's
+receptive field the chunking is invisible."""
 import types
 
 import pytest
 import torch
 import torch.nn.functional as F
 
+from conftest import load_golden
 from voicefixer_main_b200.longform import BoxcarOverlapAdd, WindowedOverlapAdd
 
-REF = "/root/reference/tools/dsp/overlapadd_boxcar.py"
 CASES = [(1000, 256, 32), (1024, 256, 32), (200, 256, 32), (256, 256, 64), (513, 256, 255), (2049, 512, 100)]
 
 
@@ -41,29 +40,31 @@ def _signal(n, batch=2):
     return torch.randn(batch, 1, n, generator=g)
 
 
-def _load_reference_class():
-    spec = importlib.util.spec_from_file_location("ref_overlapadd_boxcar", REF)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod.LambdaOverlapAdd
+def boxcar_key(n, w, m, windowed):
+    return f"boxcar_{n}_{w}_{m}_{int(windowed)}"
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not present")
+def ola_key(n, w, hop, windowed):
+    return f"ola_{n}_{w}_{hop}_{int(windowed)}"
+
+
+@pytest.fixture(scope="module")
+def reference():
+    return load_golden("reference_longform.npz")
+
+
 @pytest.mark.parametrize("n,w,m", CASES)
 @pytest.mark.parametrize("windowed", [False, True])
-def test_matches_reference_lambda_overlap_add(n, w, m, windowed):
-    Ref = _load_reference_class()
-    x = _signal(n)
-    ref_net, our_net = ToyNet(), ToyNet()
-    # the reference constructor only survives with a window name (None.type_as fails at :411); the boxcar path is
-    # then selected the way its own ola_forward does, through use_window
-    ref = Ref(nnet=ref_net, n_src=1, window_size=w, in_margin=m, window="hann", reorder_chunks=False)
-    ref.use_window = windowed
+def test_matches_reference_lambda_overlap_add(n, w, m, windowed, reference):
+    # the reference ran with window="hann" (its constructor fails on None, :411) and use_window = windowed, which
+    # selects the boxcar path the way its own ola_forward does
+    our_net = ToyNet()
     ours = BoxcarOverlapAdd(our_net, n_src=1, window_size=w, in_margin=m, window="hann" if windowed else None)
-    a, b = ref(x), ours(x)
-    assert a.shape == b.shape == (2, 1, n)
-    assert torch.equal(a, b)
-    assert sorted(ref_net.calls) == sorted(our_net.calls)          # same chunks reach the network
+    b = ours(_signal(n))
+    assert b.shape == (2, 1, n)
+    assert torch.equal(torch.from_numpy(reference[boxcar_key(n, w, m, windowed)]), b.reshape(-1)[::int(reference["stride"])])
+    calls = [tuple(c) for c in reference[boxcar_key(n, w, m, windowed) + "_calls"].tolist()]
+    assert calls == sorted(our_net.calls)                          # same chunks reach the network
 
 
 @pytest.mark.parametrize("n,w,m", CASES)
@@ -104,27 +105,20 @@ def test_plan_and_argument_checks():
 
 
 # ------------------------------------------------------------------ windowed overlap-add (tools/dsp/overlapadd.py)
-REF_OLA = "/root/reference/tools/dsp/overlapadd.py"
 OLA_CASES = [(1000, 256, None), (1024, 256, 128), (300, 256, 64), (2049, 512, 256), (777, 128, 32)]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_OLA), reason="reference tree not present")
 @pytest.mark.parametrize("n,w,hop", OLA_CASES)
 @pytest.mark.parametrize("windowed", [True, False])
-def test_windowed_ola_matches_reference(n, w, hop, windowed):
-    spec = importlib.util.spec_from_file_location("ref_overlapadd", REF_OLA)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    x = _signal(n)
-    ref_net, our_net = ToyNet(), ToyNet()
-    ref = mod.LambdaOverlapAdd(nnet=ref_net, n_src=1, window_size=w, hop_size=hop, window="hann", reorder_chunks=False)
-    ref.use_window = windowed
+def test_windowed_ola_matches_reference(n, w, hop, windowed, reference):
+    # the reference (tools/dsp/overlapadd.py) ran with window="hann" and use_window = windowed
+    our_net = ToyNet()
     ours = WindowedOverlapAdd(our_net, n_src=1, window_size=w, hop_size=hop, window="hann" if windowed else None,
                               reorder_chunks=False)
-    a, b = ref(x), ours(x)
-    assert a.shape == b.shape == (2, 1, n)
-    assert torch.equal(a, b)
-    assert ref_net.calls == our_net.calls
+    b = ours(_signal(n))
+    assert b.shape == (2, 1, n)
+    assert torch.equal(torch.from_numpy(reference[ola_key(n, w, hop, windowed)]), b.reshape(-1)[::int(reference["stride"])])
+    assert [tuple(c) for c in reference[ola_key(n, w, hop, windowed) + "_calls"].tolist()] == our_net.calls
 
 
 @pytest.mark.parametrize("n,w,hop", OLA_CASES)
