@@ -14,6 +14,7 @@
  *   vf_vocoder                    model.vocoder(mel) eval_gsr_voicefixer.py:66 (third-party voicefixer.Vocoder)
  *   vf_restore / vf_restore_host  one iteration of the segment loop of handler(), eval_gsr_voicefixer.py:49-74:
  *                                 pre -> model -> from_log -> vocoder -> peak normalise -> trim_center
+ *   vf_restore_varlen             the same over a batch of clips of different lengths (each row as if restored alone)
  *   vf_to_log / vf_from_log       tools/pytorch/pytorch_util.py:157-163
  *   vf_to_pcm16                   the int16 conversion of save_wave, tools/file/wav.py:22-24 (SURVEY.md 8(f) row 3)
  *   vf_mel                        MelScale.forward on any spectrogram, tools/pytorch/mel_scale.py:52-64
@@ -128,6 +129,14 @@ VF_API int vf_restore(vf_ctx* ctx, const float* wav, int batch, int64_t n_sample
                                         meta["unify_energy"] is set, eval_gsr_voicefixer.py:54-55 */
 VF_API int vf_restore_ex(vf_ctx* ctx, const float* wav, int batch, int64_t n_samples, float* wav_out, unsigned flags,
                          void* stream);
+/* vf_restore_ex over clips of different lengths.  wav [B, n_max] device; row b holds n_samples[b] valid samples (the rest is
+ * never read).  n_samples: HOST array of B lengths, 1024 < n_samples[b] <= n_max; checked before anything is launched
+ * (VF_EINVAL), and free for reuse as soon as the call returns.  wav_out [B, n_max] device: row b is bit-identical to
+ * vf_restore_ex of that clip alone with the same flags; samples past n_samples[b] are 0.  Plans are cached per (batch,
+ * 64-frame bucket of the longest clip), so calls whose longest clip falls in the same 0.64 s bucket share one plan and its
+ * CUDA graphs; batches above 128 clips (or above the plan budget) run as sub-batches. */
+VF_API int vf_restore_varlen(vf_ctx* ctx, const float* wav, int batch, int64_t n_max, const int64_t* n_samples,
+                             float* wav_out, unsigned flags, void* stream);
 /* Same through HOST buffers (pinned for true asynchrony).  The copies and the compute run on library-owned streams with
  * two staging buffer pairs, so back-to-back calls overlap (the H2D of call i+1 and the D2H of call i-1 run under the
  * compute of call i); `stream` only receives a wait on this call's D2H.  Contract: wav_host holds its data when the
@@ -205,7 +214,7 @@ VF_API int vf_check_errors(vf_ctx* ctx, void* stream);
  * "host_pipeline" (default 1, see vf_restore_host),
  * "validate_simt" (1: run every GEMM on the SIMT validation kernel instead of tcgen05 - tests only). */
 VF_API int vf_set_option(vf_ctx* ctx, const char* key, int value);
-/* Plans are cached per (path, batch, frames); the cache is bounded (see "plan_cache_mb").  A batch whose plan would not fit
+/* Plans are cached per (path, batch, frames) - frames rounded up to 64 for vf_restore_varlen; the cache is bounded (see "plan_cache_mb").  A batch whose plan would not fit
  * the budget is processed in sub-batches through a smaller plan (same results: rows are independent); the *_stages accessors
  * then only see the last sub-batch. */
 VF_API int vf_plan_cache_info(vf_ctx* ctx, int* n_plans, size_t* bytes, size_t* budget, int64_t* evicted);

@@ -10,6 +10,28 @@ namespace vf {
 __device__ __forceinline__ float lrelu(float a, float slope) { return a > 0.f ? a : a * slope; }
 
 // ---------------------------------------------------------------------------------------------
+// Per-clip table of a varlen call (kernels.cuh VarlenImage): one thread per clip, the lengths by value.
+__global__ void varlen_setup_kernel(const __grid_constant__ VarlenSetupParams p) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= p.batch) return;
+  VarlenImage r;
+  r.n = (int)p.n[b];
+  r.T = 1 + r.n / p.hop;
+  r.Tp = (r.T + 63) / 64 * 64;
+  for (int l = 0; l < 7; ++l) r.unet_rows[l] = (r.Tp >> l) * ((p.W0 >> l) + 1);
+  r.voc_len[0] = r.T + r.T % 2 + p.tail_base;
+  for (int s = 0; s < 8; ++s) r.voc_len[s + 1] = s < p.num_stages ? r.voc_len[s] * p.scales[s] : 0;
+  r.L = r.voc_len[p.num_stages];
+  r.skip = (r.L - r.n) / 2;
+  r.pad_[0] = r.pad_[1] = r.pad_[2] = 0;
+  p.out[b] = r;
+}
+cudaError_t launch_varlen_setup(const VarlenSetupParams& p, cudaStream_t stream) {
+  varlen_setup_kernel<<<(p.batch + 127) / 128, 128, 0, stream>>>(p);
+  return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128) unet_first_kernel(UnetFirstParams p) {
   const size_t pix = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int Wp = p.W + 1;
@@ -19,8 +41,10 @@ __global__ void __launch_bounds__(128) unet_first_kernel(UnetFirstParams p) {
   const int f = (int)(pix - row * Wp);
   const int t = (int)(row % p.Tp);
   const int b = (int)(row / p.Tp);
+  int T = p.T, Tp = p.Tp;          // frames / padded frames of this clip (T is also the row stride of logmel)
+  if (p.vl) { T = p.vl[b].T; Tp = p.vl[b].Tp; }
   float out_a[32], out_r[32];
-  if (f == p.W) {
+  if (f == p.W || t >= Tp) {       // pad column, or past this clip's padded frames: zeros
 #pragma unroll
     for (int c = 0; c < 32; ++c) { out_a[c] = 0.f; out_r[c] = 0.f; }
   } else {
@@ -32,8 +56,8 @@ __global__ void __launch_bounds__(128) unet_first_kernel(UnetFirstParams p) {
       for (int dw = 0; dw < 3; ++dw) {
         const int tt = t + dh - 1, ff = f + dw - 1;
         float v = 0.f;
-        if (tt >= 0 && tt < p.Tp && ff >= 0 && ff < p.W) {
-          const float x = tt < p.T ? __ldg(p.logmel + ((size_t)b * p.T + tt) * p.in_ld + ff) : 0.f;
+        if (tt >= 0 && tt < Tp && ff >= 0 && ff < p.W) {
+          const float x = tt < T ? __ldg(p.logmel + ((size_t)b * p.T + tt) * p.in_ld + ff) : 0.f;
           if (dh == 1 && dw == 1) xc = x;
           v = lrelu(fmaf(x, p.bn1_scale, p.bn1_shift), p.slope);
         }
@@ -77,7 +101,7 @@ __global__ void __launch_bounds__(256) pool_kernel(PoolParams p) {
   const int h = (opix / Wpo) % Ho;
   const int b = opix / ((size_t)Wpo * Ho);
   float v[8], a[8];
-  if (w == Wpo - 1) {
+  if (w == Wpo - 1 || (p.vl && (int)(opix - (size_t)b * Wpo * Ho) >= p.vl[b].unet_rows[p.vl_level])) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) { v[i] = 0.f; a[i] = 0.f; }
   } else {
@@ -146,7 +170,15 @@ __global__ void __launch_bounds__(256) voc_condition_kernel(VocCondParams p) {
   const int tv = (idx >> 4) % p.Tv;
   const int b = (idx >> 4) / p.Tv;
   float c[8];
-  if (tv >= p.T) {
+  int T = p.T;                       // this clip's frames (p.T is also the row stride of mel)
+  if (p.vl) {
+    T = p.vl[b].T;
+    if (tv >= p.vl[b].voc_len[0]) T = -1;
+  }
+  if (T < 0) {                       // past this clip's conditioning rows: zeros
+#pragma unroll
+    for (int i = 0; i < 8; ++i) c[i] = 0.f;
+  } else if (tv >= T) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) c[i] = p.tail_value;
   } else {
@@ -165,11 +197,13 @@ __global__ void __launch_bounds__(256) voc_condition_kernel(VocCondParams p) {
 }
 // One CTA per clip, fixed reduction order: the scale amp_to_original_f applies (and with it every output sample) is
 // reproducible run to run (a multi-CTA atomicAdd version differed in the last bits between identical calls).
-__global__ void __launch_bounds__(256) band_energy_kernel(const float* tgt, const float* logest, int T, float* sums) {
+__global__ void __launch_bounds__(256) band_energy_kernel(const float* tgt, const float* logest, int T, float* sums,
+                                                          const VarlenImage* vl) {
   __shared__ float sh[2][8];
   const int b = blockIdx.x;
+  const int Tb = vl ? vl[b].T : T;   // frames of this clip; T stays the row stride
   float st = 0.f, se = 0.f;
-  for (int i = threadIdx.x; i < T * 20; i += 256) {
+  for (int i = threadIdx.x; i < Tb * 20; i += 256) {
     const size_t idx = ((size_t)b * T + i / 20) * 128 + 5 + i % 20;
     st += __ldg(tgt + idx);
     se += exp10f(fminf(__ldg(logest + idx), 5.f));
@@ -189,8 +223,8 @@ __global__ void __launch_bounds__(256) band_energy_kernel(const float* tgt, cons
   }
 }
 cudaError_t launch_band_energy(const float* mel_target_lin, const float* logmel_est, int batch, int T, float* sums,
-                               cudaStream_t stream) {
-  band_energy_kernel<<<batch, 256, 0, stream>>>(mel_target_lin, logmel_est, T, sums);
+                               cudaStream_t stream, const VarlenImage* vl) {
+  band_energy_kernel<<<batch, 256, 0, stream>>>(mel_target_lin, logmel_est, T, sums, vl);
   return cudaGetLastError();
 }
 
@@ -235,7 +269,7 @@ cudaError_t launch_voc_condition(const VocCondParams& p, cudaStream_t stream) {
 }
 
 // ---------------------------------------------------------------------------------------------
-__global__ void reflect_fill_kernel(PlanePtr pl, int batch, int L, int C, int pad) {
+__global__ void reflect_fill_kernel(PlanePtr pl, int batch, int Lmax, int C, int pad, const VarlenImage* vl, int vl_stage) {
   const int cg = C / 8;
   const size_t total = (size_t)batch * 2 * pad * cg;
   const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -243,17 +277,19 @@ __global__ void reflect_fill_kernel(PlanePtr pl, int batch, int L, int C, int pa
   const int g = idx % cg;
   const int j = (idx / cg) % (2 * pad);
   const int b = idx / ((size_t)cg * 2 * pad);
+  const int L = vl ? vl[b].voc_len[vl_stage] : Lmax;     // this clip's length; Lmax sets the row pitch
   int dst, src;
   if (j < pad) { dst = j; src = 2 * pad - j; }
   else { const int i = j - pad; dst = L + pad + i; src = L - 2 - i + pad; }
-  const size_t rows = (size_t)L + 2 * pad;
+  const size_t rows = (size_t)Lmax + 2 * pad;
   const size_t d = ((size_t)b * rows + dst) * C + g * 8, s = ((size_t)b * rows + src) * C + g * 8;
   *reinterpret_cast<uint4*>(pl.hi + d) = *reinterpret_cast<const uint4*>(pl.hi + s);
   *reinterpret_cast<uint4*>(pl.lo + d) = *reinterpret_cast<const uint4*>(pl.lo + s);
 }
-cudaError_t launch_reflect_fill(PlanePtr planes, int batch, int L, int C, int pad, cudaStream_t stream) {
+cudaError_t launch_reflect_fill(PlanePtr planes, int batch, int L, int C, int pad, cudaStream_t stream, const VarlenImage* vl,
+                                int vl_stage) {
   const size_t total = (size_t)batch * 2 * pad * (C / 8);
-  reflect_fill_kernel<<<(unsigned)((total + 127) / 128), 128, 0, stream>>>(planes, batch, L, C, pad);
+  reflect_fill_kernel<<<(unsigned)((total + 127) / 128), 128, 0, stream>>>(planes, batch, L, C, pad, vl, vl_stage);
   return cudaGetLastError();
 }
 
@@ -335,13 +371,16 @@ __global__ void __launch_bounds__(TAIL_THREADS) voc_tail_kernel(VocTailParams p)
     }
   }
   float mag = 0.f;
+  const long Lb = p.vl ? p.vl[b].L : p.L;     // this clip's samples (p.L is the row pitch)
 #pragma unroll
   for (int o = 0; o < TAIL_RT; ++o) {
     const long t = t0 + r0 + o;
-    if (t < p.L) {
+    if (t < Lb) {
       const float y = p.tanh_out ? tanhf(acc[o] + p.bias) : acc[o] + p.bias;
       p.wav[(size_t)b * p.L + t] = y;
       mag = fmaxf(mag, fabsf(y));
+    } else if (t < p.L) {
+      p.wav[(size_t)b * p.L + t] = 0.f;
     }
   }
 #pragma unroll
@@ -376,8 +415,13 @@ __global__ void finalize_kernel(FinalizeParams p) {
   const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
   const int b = blockIdx.y;
   if (i >= p.n) return;
+  long skip = p.skip;
+  if (p.vl) {                        // clip of its own length: its own trim offset, zeros past its samples
+    if (i >= p.vl[b].n) { p.out[(size_t)b * p.out_ld + p.out_off + i] = 0.f; return; }
+    skip = p.vl[b].skip;
+  }
   const float peak = __uint_as_float(p.peak_bits[b]);
-  float v = p.wav[(size_t)b * p.L + p.skip + i];
+  float v = p.wav[(size_t)b * p.L + skip + i];
   if (peak > 1.0f) v = v / peak;
   p.out[(size_t)b * p.out_ld + p.out_off + i] = v;
 }

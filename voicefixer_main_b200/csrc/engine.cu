@@ -10,6 +10,8 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdarg>
+#include <cstddef>
+#include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -87,7 +89,7 @@ struct Op {
   UnetFirstParams first;
   PoolParams pool;
   VocCondParams cond;
-  struct { PlanePtr pl; int batch, L, C, pad; } refl;
+  struct { PlanePtr pl; int batch, L, C, pad; const VarlenImage* vl; int vl_stage; } refl;
   VocTailParams tail;
   FinalizeParams fin;
   struct { void* p; size_t bytes; } ms;
@@ -114,7 +116,9 @@ struct UnetW {
   float head_b = 0;
 };
 
-enum PlanKind { PLAN_GSR = 0, PLAN_SSR = 1 };
+// PLAN_GSR_VARLEN: the GSR chain over clips of different lengths (vf_restore_varlen), keyed by the 64-frame bucket of the
+// longest clip; its kernels take the per-clip lengths from the plan's VarlenImage table
+enum PlanKind { PLAN_GSR = 0, PLAN_SSR = 1, PLAN_GSR_VARLEN = 2 };
 
 struct Plan {
   int kind = PLAN_GSR;
@@ -138,6 +142,7 @@ struct Plan {
   float* d_logmel_out = nullptr; // [B, T, 128]
   float* d_voc_wav = nullptr;    // [B, L]
   float* d_band = nullptr;       // [B][2] low-band energy sums (unify_energy)
+  VarlenImage* d_vl = nullptr;   // [B] per-clip lengths of the current call (PLAN_GSR_VARLEN only)
   unsigned int* d_peak = nullptr;
   long L = 0;
   // SSR plans (unet_v2 + ISTFT)
@@ -942,6 +947,17 @@ void set_out_a(GemmEpilogue& e, const Planes& pl, int c_off, const float* scale,
   e.act = act;
   e.slope = slope;
 }
+// Column `byte_offset` of the per-clip table (null on the equal-length path): output rows at or past it are written as zeros
+const int* vl_col(const VarlenImage* vl, size_t byte_offset) {
+  return vl ? reinterpret_cast<const int*>(reinterpret_cast<const char*>(vl) + byte_offset) : nullptr;
+}
+void set_vl_rows(GemmEpilogue& e, const int* col) {
+  e.vl_rows = col;
+  e.vl_stride = VARLEN_STRIDE;
+}
+size_t vl_unet(int level) { return offsetof(VarlenImage, unet_rows) + sizeof(int) * level; }
+size_t vl_voc(int stage) { return offsetof(VarlenImage, voc_len) + sizeof(int) * stage; }
+
 std::vector<GemmTap> taps3x3(int Wp, int cin) {
   std::vector<GemmTap> t;
   for (int kh = 0; kh < 3; ++kh)
@@ -950,7 +966,7 @@ std::vector<GemmTap> taps3x3(int Wp, int cin) {
 }
 
 struct Level {
-  int H, W, Wp, C, rows;
+  int lvl, H, W, Wp, C, rows;
   float* raw[2];
   Planes aX, aT, cat_r, cat_a, P_r, P_a;   // P_* : pooled output of this level (input of the next)
   float* P_raw = nullptr;
@@ -973,10 +989,11 @@ int build_unet(vf_ctx* ctx, Builder& b, Plan* plan, const UnetW& U, const UnetGe
   std::vector<Op>& ops = plan->unet;
   const int terms = ctx->unet_terms;
   const float S = 0.01f;   // LeakyReLU slope, modules.py:265-266
+  const VarlenImage* vl = plan->d_vl;
   Level lv[7];
   for (int l = 0; l < 7; ++l) {
     Level& L = lv[l];
-    L.H = Tp >> l; L.W = G.W0 >> l; L.Wp = L.W + 1; L.C = l < 6 ? ENC_C[l] : 384; L.rows = L.H * L.Wp;
+    L.lvl = l; L.H = Tp >> l; L.W = G.W0 >> l; L.Wp = L.W + 1; L.C = l < 6 ? ENC_C[l] : 384; L.rows = L.H * L.Wp;
     L.raw[0] = b.alloc<float>((size_t)B * L.rows * L.C);
     L.raw[1] = b.alloc<float>((size_t)B * L.rows * L.C);
     L.aX = b.planes(B, L.rows, L.C);
@@ -1000,6 +1017,7 @@ int build_unet(vf_ctx* ctx, Builder& b, Plan* plan, const UnetW& U, const UnetGe
     b.label = tag + ".conv1";
     GemmEpilogue e = epi_plain(L.rows, L.Wp, w.cout, L.rows);
     set_out_a(e, L.aT, 0, w.bn2.scale, w.bn2.shift, ACT_LRELU, S);
+    set_vl_rows(e, vl_col(vl, vl_unet(L.lvl)));
     b.gemm(ops, w.conv1, ASrc{in, L.rows, 0}, nullptr, taps3x3(L.Wp, w.cin), e, B, terms);
   };
   // conv2 of a block: aT (+ 1x1 shortcut of sc_src) (+ residual) -> outputs set by the caller
@@ -1013,6 +1031,7 @@ int build_unet(vf_ctx* ctx, Builder& b, Plan* plan, const UnetW& U, const UnetGe
     }
     e.resid = resid;
     e.resid_ld = w.cout;
+    set_vl_rows(e, vl_col(vl, vl_unet(L.lvl)));
     b.label = tag + (sc_src ? ".conv2+sc" : ".conv2");
     b.gemm(ops, w.conv2, ASrc{L.aT, L.rows, 0}, sc_src ? &s1 : nullptr, taps, e, B, terms);
   };
@@ -1034,7 +1053,7 @@ int build_unet(vf_ctx* ctx, Builder& b, Plan* plan, const UnetW& U, const UnetGe
         f.bn1_scale = U.first_bn1_scale; f.bn1_shift = U.first_bn1_shift;
         f.w1 = U.d_first_w1; f.bn2_scale = w.bn2.scale; f.bn2_shift = w.bn2.shift;
         f.w_sc = U.d_first_wsc; f.b_sc = U.d_first_bsc; f.slope = S;
-        f.a2 = L.aT.p; f.sc_raw = L.raw[0]; f.err = ctx->d_err;
+        f.a2 = L.aT.p; f.sc_raw = L.raw[0]; f.err = ctx->d_err; f.vl = vl;
         ops.push_back(op);
         resid = L.raw[0];      // precomputed shortcut(x) acts as the residual
         cur = 0;
@@ -1071,6 +1090,7 @@ int build_unet(vf_ctx* ctx, Builder& b, Plan* plan, const UnetW& U, const UnetGe
     p.in = L.raw[cur]; p.batch = B; p.H = L.H; p.Wp = L.Wp; p.C = L.C; p.Wpo = (L.W >> 1) + 1;
     p.out_r = L.P_r.p; p.out_a = L.P_a.p; p.out_raw = L.P_raw;
     p.a_scale = nx.bn1.scale; p.a_shift = nx.bn1.shift; p.slope = S; p.err = ctx->d_err;
+    p.vl = vl; p.vl_level = l + 1;
     ops.push_back(op);
   }
   // ---------------- bottleneck (conv_block7, identity shortcut) -> decoder_block1.bn1 + ReLU
@@ -1093,6 +1113,7 @@ int build_unet(vf_ctx* ctx, Builder& b, Plan* plan, const UnetW& U, const UnetGe
       e.map = MAP_CONVT2D; e.rows_in = Lin.rows; e.Wp = Lin.Wp; e.cout = cout; e.out_img_rows = L.rows;
       e.out_rows_valid = L.rows;
       e.ct_out_wp = L.Wp;      // 2 * Lin.Wp (time-only prune, modules.py:209) or 2 * Lin.Wp - 1 (both=True, modules.py:207-208)
+      set_vl_rows(e, vl_col(vl, vl_unet(L.lvl)));
       const ConvBlockW& blk = U.dec[k][0];
       e.out_r = OutPlane{L.cat_r.p.hi, L.cat_r.p.lo, 2 * L.C, 0};
       set_out_a(e, L.cat_a, 0, blk.bn1.scale, blk.bn1.shift, ACT_LRELU, S);
@@ -1131,6 +1152,7 @@ int build_unet(vf_ctx* ctx, Builder& b, Plan* plan, const UnetW& U, const UnetGe
       GemmEpilogue e = epi_plain(L.rows, L.Wp, 32, L.rows);
       e.head_w = U.d_head_w; e.head_b = U.head_b;
       e.head_in = G.head_in; e.head_out = G.head_out; e.head_T = T;
+      e.vl_head_T = vl_col(vl, offsetof(VarlenImage, T));      // conv2 sets vl_stride
       conv2(U.post, L, nullptr, L.raw[cur], e);
     }
   }
@@ -1144,6 +1166,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
   const int terms = ctx->voc_terms;
   std::vector<Op>& ops = plan->vocoder;
   const int CC = c.voc_cond_channels;
+  const VarlenImage* vl = plan->d_vl;
 
   Planes cond = b.planes(B, Tv, 128);
   Planes c0 = b.planes(B, Tv, CC), c1 = b.planes(B, Tv, CC);
@@ -1156,7 +1179,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
     memset(&p, 0, sizeof p);
     p.mel = plan->d_logmel_out; p.is_log = 1; p.batch = B; p.T = T; p.Tv = Tv; p.weight = ctx->d_melw;
     p.amp_floor = c.voc_amp_floor; p.ref_db = c.voc_ref_db; p.min_db = c.voc_min_db; p.tail_value = c.voc_tail_value;
-    p.out = cond.p;
+    p.out = cond.p; p.vl = vl;
     plan->cond_op = (int)ops.size();
     ops.push_back(op);
   }
@@ -1173,15 +1196,18 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
     e.out_row0 = last ? 3 : 0;
     e.bias = ctx->voc_cond[i].bias;
     set_out_a(e, dst, 0, nullptr, nullptr, ACT_ELU, 0.f);
+    set_vl_rows(e, vl_col(vl, vl_voc(0)));
     b.label = "voc.cond" + std::to_string(i);
     b.gemm(ops, ctx->voc_cond[i], ASrc{cur, Tv, 0}, nullptr, taps1d(3, 1, cur.C, true), e, B, terms);
     cur = dst;
   }
-  { Op op; op.kind = OP_REFLECT; op.refl.pl = cpad.p; op.refl.batch = B; op.refl.L = Tv; op.refl.C = CC; op.refl.pad = 3; ops.push_back(op); }
+  { Op op; op.kind = OP_REFLECT; op.refl.pl = cpad.p; op.refl.batch = B; op.refl.L = Tv; op.refl.C = CC; op.refl.pad = 3;
+    op.refl.vl = vl; op.refl.vl_stage = 0; ops.push_back(op); }
   {
     GemmEpilogue e = epi_plain(Tv, 0, c.voc_channels, Tv);
     e.bias = ctx->voc_stem.bias;
     set_out_a(e, stem, 0, nullptr, nullptr, ACT_LRELU, c.voc_stage_slope);
+    set_vl_rows(e, vl_col(vl, vl_voc(0)));
     b.label = "voc.stem";
     b.gemm(ops, ctx->voc_stem, ASrc{cpad, Tv + 6, 0}, nullptr, taps1d(7, 1, CC, false), e, B, terms);
   }
@@ -1190,6 +1216,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
   int cin = c.voc_channels;
   for (int s = 0; s < c.voc_num_stages; ++s) {
     const int sc = c.voc_scales[s], cout = cin / 2;
+    if (vl && sc > 24) return fail(ctx, VF_EINVAL, "varlen vocoder: up-sampling scale %d above 24 (one flag bit per phase)", sc);
     const long L = Lprev * sc;
     const bool last_stage = s == c.voc_num_stages - 1;
     // C = 64 stacks in the hi-only mode: one kernel per residual pair (pair_tc.cu), the intermediate h stays in shared
@@ -1219,6 +1246,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
       if (ar) e.out_ar = ar;
       else e.out_r = OutPlane{xr[0].p.hi, xr[0].p.lo, cout, 0};
       set_out_a(e, xa, 0, nullptr, nullptr, ACT_LRELU, c.voc_res_slope);
+      set_vl_rows(e, vl_col(vl, vl_voc(s + 1)));
       std::vector<GemmTap> taps = {GemmTap{0, 0, 0, 0, cin}, GemmTap{-1, 0, 0, 0, cin}};
       b.label = "voc.up" + std::to_string(s);
       b.gemm(ops, ctx->voc_up[s], ASrc{prev, (int)Lprev, 0}, nullptr, taps, e, B, terms);
@@ -1286,6 +1314,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
         pp.slope_h = c.voc_res_slope;
         pp.slope_out = last ? c.voc_stage_slope : c.voc_res_slope;
         pp.err = ctx->d_err;
+        pp.vl_len = vl_col(vl, vl_voc(s + 1)); pp.vl_stride = VARLEN_STRIDE;
         op.flops = 2.0 * 2.0 * (double)B * L * cout * 3.0 * cout;
         op.exec_flops = 2.0 * 2.0 * (double)B * pp.tiles_per_img * GEMM_BM * cout * 3.0 * cout;
         op.bytes = ar ? (double)B * L * cout * (2 + 2 + (last ? 0 : 2) + 2)    // act in (operand and residual), r in, r out, act out
@@ -1300,6 +1329,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
         GemmEpilogue e = epi_plain((int)L, 0, cout, (int)L);
         e.bias = ctx->voc_res_a[s][i].bias;
         set_out_a(e, ha, 0, nullptr, nullptr, ACT_LRELU, c.voc_res_slope);
+        set_vl_rows(e, vl_col(vl, vl_voc(s + 1)));
         b.label = "voc.res" + std::to_string(s) + "." + std::to_string(i) + ".a";
         b.gemm(ops, ctx->voc_res_a[s][i], ASrc{xa, (int)L, 0}, nullptr, taps1d(3, dil, cout, true), e, B, terms);
       }
@@ -1313,6 +1343,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
           else e.out_r = OutPlane{xr[1 - curx].p.hi, xr[1 - curx].p.lo, cout, 0};
         }
         set_out_a(e, dst, 0, nullptr, nullptr, ACT_LRELU, last ? c.voc_stage_slope : c.voc_res_slope);
+        set_vl_rows(e, vl_col(vl, vl_voc(s + 1)));
         b.label = "voc.res" + std::to_string(s) + "." + std::to_string(i) + ".b";
         std::vector<GemmTap> taps = taps1d(3, 1, cout, true);
         ASrc xsrc{xr[curx], (int)L, 0};
@@ -1335,7 +1366,8 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
       }
     }
     if (last_stage) {
-      { Op op; op.kind = OP_REFLECT; op.refl.pl = tail_in.p; op.refl.batch = B; op.refl.L = (int)L; op.refl.C = cout; op.refl.pad = 3; ops.push_back(op); }
+      { Op op; op.kind = OP_REFLECT; op.refl.pl = tail_in.p; op.refl.batch = B; op.refl.L = (int)L; op.refl.C = cout; op.refl.pad = 3;
+        op.refl.vl = vl; op.refl.vl_stage = c.voc_num_stages; ops.push_back(op); }
       plan->L = L;
       plan->d_voc_wav = b.alloc<float>((size_t)B * L);
       plan->d_peak = b.alloc<unsigned int>(B);
@@ -1345,7 +1377,7 @@ int build_vocoder(vf_ctx* ctx, Builder& b, Plan* plan) {
       VocTailParams& p = op.tail;
       memset(&p, 0, sizeof p);
       p.in = tail_in.p; p.batch = B; p.L = (int)L; p.C = cout; p.terms = terms; p.w = ctx->d_tail_w; p.bias = ctx->tail_b;
-      p.wav = plan->d_voc_wav; p.peak_bits = plan->d_peak; p.tanh_out = c.voc_tail_tanh;
+      p.wav = plan->d_voc_wav; p.peak_bits = plan->d_peak; p.tanh_out = c.voc_tail_tanh; p.vl = vl;
       ops.push_back(op);
     }
     prev = (fused && cura) ? xa2 : xa;
@@ -1418,7 +1450,7 @@ int get_plan(vf_ctx* ctx, int kind, int batch, int frames, Plan** out) {
   auto it = ctx->plans.find(key);
   if (it != ctx->plans.end()) { it->second->last_use = ++ctx->use_clock; *out = it->second.get(); return VF_OK; }
   if (!ctx->loaded) return fail(ctx, VF_ESTATE, "weights not loaded");
-  if (kind == PLAN_GSR && !(ctx->gsr.loaded && ctx->voc_loaded))
+  if ((kind == PLAN_GSR || kind == PLAN_GSR_VARLEN) && !(ctx->gsr.loaded && ctx->voc_loaded))
     return fail(ctx, VF_ESTATE, "this entry point needs the analysis module (generator.analysis_module.*) and the vocoder (vocoder.*) weights");
   if (kind == PLAN_SSR && !ctx->ssr.loaded)
     return fail(ctx, VF_ESTATE, "this entry point needs the unet_v2 weights (generator.unet.*)");
@@ -1438,7 +1470,8 @@ int get_plan(vf_ctx* ctx, int kind, int batch, int frames, Plan** out) {
   plan->kind = kind; plan->batch = batch; plan->T = frames;
   Builder b{ctx, plan.get()};
   int rc = VF_OK;
-  if (kind == PLAN_GSR) {
+  if (kind == PLAN_GSR || kind == PLAN_GSR_VARLEN) {
+    if (kind == PLAN_GSR_VARLEN) plan->d_vl = b.alloc<VarlenImage>(batch);     // before the builders: their ops point into it
     const size_t mel_n = (size_t)batch * frames * 128;
     plan->d_mel = b.alloc<float>(mel_n);
     plan->d_logmel_in = b.alloc<float>(mel_n);
@@ -1566,7 +1599,7 @@ int run_ops(vf_ctx* ctx, std::vector<Op>& ops, cudaStream_t st) {
       case OP_FIRST: e = launch_unet_first(op.first, st); break;
       case OP_POOL: e = launch_pool(op.pool, st); break;
       case OP_COND: e = launch_voc_condition(op.cond, st); break;
-      case OP_REFLECT: e = launch_reflect_fill(op.refl.pl, op.refl.batch, op.refl.L, op.refl.C, op.refl.pad, st); break;
+      case OP_REFLECT: e = launch_reflect_fill(op.refl.pl, op.refl.batch, op.refl.L, op.refl.C, op.refl.pad, st, op.refl.vl, op.refl.vl_stage); break;
       case OP_TAIL: e = launch_voc_tail(op.tail, st); break;
       case OP_FINALIZE: e = launch_finalize(op.fin, st); break;
       case OP_MEMSET32: e = cudaMemsetAsync(op.ms.p, 0, op.ms.bytes, st); break;
@@ -1622,12 +1655,13 @@ int run_chain(vf_ctx* ctx, Plan* plan, int slot, cudaStream_t st, int64_t n_laun
 
 int frames_of(vf_ctx* ctx, long n) { return 1 + (int)(n / ctx->cfg.hop); }
 
+// vl (varlen plans): n is the row stride of wav, `frames` the plan's frames; each clip's own lengths come from the table
 int run_frontend(vf_ctx* ctx, const float* wav, int batch, long n, float* mel, float* logmel, float* sp, float* co,
-                 float* si, cudaStream_t st) {
+                 float* si, cudaStream_t st, const VarlenImage* vl = nullptr, int frames = 0) {
   if (n <= 1024) return fail(ctx, VF_EINVAL, "reflect padding needs more than n_fft/2 = 1024 samples (got %ld)", n);
   FrontendParams p;
   memset(&p, 0, sizeof p);
-  p.wav = wav; p.n = n; p.batch = batch; p.T = frames_of(ctx, n);
+  p.wav = wav; p.n = n; p.batch = batch; p.T = vl ? frames : frames_of(ctx, n); p.vl = vl;
   p.window = ctx->d_window; p.tw1024 = ctx->d_tw1024; p.tw2048 = ctx->d_tw2048;
   p.fb_f0 = ctx->d_fb_f0; p.fb_len = ctx->d_fb_len; p.fb_ofs = ctx->d_fb_ofs; p.fb_val = ctx->d_fb_val;
   p.sp_out = sp; p.cos_out = co; p.sin_out = si; p.mel_out = mel; p.logmel_out = logmel;
@@ -1817,10 +1851,13 @@ VF_API int vf_vocoder(vf_ctx* ctx, const float* mel_lin, int batch, int frames, 
   return plan_exit(ctx, plan, st);
 }
 
-static int restore_impl(vf_ctx* ctx, const float* wav, int batch, int64_t n, float* wav_out, unsigned flags, cudaStream_t st) {
-  const int frames = frames_of(ctx, (long)n);
+// lens == null: every clip has n samples.  Else clip b has lens[b] samples (1024 < lens[b] <= n, checked by the caller), n is the
+// row stride of wav and wav_out, and `frames` the 64-frame bucket of the longest clip (the varlen plan's key).
+static int restore_impl(vf_ctx* ctx, const float* wav, int batch, int64_t n, float* wav_out, unsigned flags, cudaStream_t st,
+                        const int64_t* lens = nullptr, int bucket = 0) {
+  const int frames = lens ? bucket : frames_of(ctx, (long)n);
   Plan* plan;
-  int rc = get_plan(ctx, PLAN_GSR, batch, frames, &plan);
+  int rc = get_plan(ctx, lens ? PLAN_GSR_VARLEN : PLAN_GSR, batch, frames, &plan);
   if (rc) return rc;
   if (ctx->op_timing) ctx->prof.clear();
   rc = plan_enter(ctx, plan, st);
@@ -1831,7 +1868,18 @@ static int restore_impl(vf_ctx* ctx, const float* wav, int batch, int64_t n, flo
       if (!e) CK(cudaEventCreate(&e));
     CK(cudaEventRecord(ctx->ev[0], st));
   }
-  rc = run_frontend(ctx, wav, batch, (long)n, plan->d_mel, plan->d_logmel_in, nullptr, nullptr, nullptr, st);
+  if (lens) {     // the per-clip table of this call: a plain launch ahead of the frontend and the captured chain
+    VarlenSetupParams vp;
+    memset(&vp, 0, sizeof vp);
+    vp.batch = batch; vp.W0 = 127; vp.hop = ctx->cfg.hop; vp.tail_base = ctx->cfg.voc_tail_base;
+    vp.num_stages = ctx->cfg.voc_num_stages;
+    for (int s = 0; s < 8; ++s) vp.scales[s] = ctx->cfg.voc_scales[s];
+    vp.out = plan->d_vl;
+    for (int b = 0; b < batch; ++b) vp.n[b] = (long long)lens[b];
+    CK(launch_varlen_setup(vp, st));
+    ctx->launches++;
+  }
+  rc = run_frontend(ctx, wav, batch, (long)n, plan->d_mel, plan->d_logmel_in, nullptr, nullptr, nullptr, st, plan->d_vl, frames);
   if (rc) return rc;
   if (tm) CK(cudaEventRecord(ctx->ev[1], st));
   const bool unify = (flags & VF_RESTORE_UNIFY_ENERGY) != 0;
@@ -1846,7 +1894,7 @@ static int restore_impl(vf_ctx* ctx, const float* wav, int batch, int64_t n, flo
     cop.cond.band_sums = nullptr;
     if (unify) {
       CK(cudaMemsetAsync(plan->d_band, 0, 2 * (size_t)batch * sizeof(float), s));
-      CK(launch_band_energy(plan->d_mel, plan->d_logmel_out, batch, frames, plan->d_band, s));
+      CK(launch_band_energy(plan->d_mel, plan->d_logmel_out, batch, frames, plan->d_band, s, plan->d_vl));
       ctx->launches++;
       cop.cond.band_sums = plan->d_band;
     }
@@ -1859,9 +1907,9 @@ static int restore_impl(vf_ctx* ctx, const float* wav, int batch, int64_t n, flo
   FinalizeParams f;
   memset(&f, 0, sizeof f);
   const long d = plan->L - (long)n;
-  if (d < 0 || d == 1) return fail(ctx, VF_EINVAL, "vocoder output length %ld incompatible with input %ld (trim_center)", plan->L, (long)n);
-  f.wav = plan->d_voc_wav; f.peak_bits = plan->d_peak; f.batch = batch; f.L = plan->L; f.n = (long)n; f.skip = d / 2;
-  f.out = wav_out; f.out_ld = (long)n; f.out_off = 0;
+  if (!lens && (d < 0 || d == 1)) return fail(ctx, VF_EINVAL, "vocoder output length %ld incompatible with input %ld (trim_center)", plan->L, (long)n);
+  f.wav = plan->d_voc_wav; f.peak_bits = plan->d_peak; f.batch = batch; f.L = plan->L; f.n = (long)n; f.skip = lens ? 0 : d / 2;
+  f.out = wav_out; f.out_ld = (long)n; f.out_off = 0; f.vl = plan->d_vl;
   CK(launch_finalize(f, st));
   ctx->launches++;
   if (tm) { CK(cudaEventRecord(ctx->ev[4], st)); ctx->ev_valid = true; }
@@ -1876,6 +1924,33 @@ VF_API int vf_restore_ex(vf_ctx* ctx, const float* wav, int batch, int64_t n, fl
   const int cb = choose_sub_batch(ctx, PLAN_GSR, batch, frames_of(ctx, (long)n));
   for (int off = 0; off < batch; off += cb) {
     rc = restore_impl(ctx, wav + (size_t)off * n, std::min(cb, batch - off), n, wav_out + (size_t)off * n, flags, (cudaStream_t)stream);
+    if (rc) return rc;
+  }
+  return VF_OK;
+}
+
+VF_API int vf_restore_varlen(vf_ctx* ctx, const float* wav, int batch, int64_t n_max, const int64_t* n_samples, float* wav_out,
+                             unsigned flags, void* stream) {
+  int rc = check_ready(ctx);
+  if (rc) return rc;
+  if (!wav || !wav_out || !n_samples || batch <= 0) return fail(ctx, VF_EINVAL, "vf_restore_varlen: bad arguments");
+  if (flags & ~(unsigned)VF_RESTORE_UNIFY_ENERGY) return fail(ctx, VF_EINVAL, "vf_restore_varlen: unknown flag bits 0x%x", flags);
+  if (n_max > (int64_t)INT32_MAX / 2) return fail(ctx, VF_EINVAL, "vf_restore_varlen: n_max %ld too large", (long)n_max);
+  // every length is checked before anything is launched
+  int64_t longest = 0;
+  for (int b = 0; b < batch; ++b) {
+    if (n_samples[b] <= 1024 || n_samples[b] > n_max)
+      return fail(ctx, VF_EINVAL, "vf_restore_varlen: clip %d has %ld samples; need 1024 < n <= n_max = %ld (reflect padding needs "
+                  "more than n_fft/2 samples)", b, (long)n_samples[b], (long)n_max);
+    longest = std::max(longest, n_samples[b]);
+  }
+  // one plan per (batch, 64-frame bucket of the longest clip): every call whose longest clip is in the same 0.64 s bucket
+  // reuses it and its CUDA graphs
+  const int bucket = round_up(frames_of(ctx, (long)longest), 64);
+  const int cb = std::min(choose_sub_batch(ctx, PLAN_GSR_VARLEN, batch, bucket), VF_VARLEN_MAX_CLIPS);
+  for (int off = 0; off < batch; off += cb) {
+    rc = restore_impl(ctx, wav + (size_t)off * n_max, std::min(cb, batch - off), n_max, wav_out + (size_t)off * n_max, flags,
+                      (cudaStream_t)stream, n_samples + off, bucket);
     if (rc) return rc;
   }
   return VF_OK;

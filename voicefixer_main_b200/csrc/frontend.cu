@@ -21,9 +21,21 @@ __global__ void __launch_bounds__(256) frontend_kernel(FrontendParams p) {
   __shared__ float2 buf1[1024];
   const int t = blockIdx.x, b = blockIdx.y, tid = threadIdx.x;
   const float* x = p.wav + (size_t)b * p.n;
+  long n = p.n;
+  if (p.vl) {                    // clip of its own length in a wider batch: reflect at its end, zeros past its frames
+    n = p.vl[b].n;
+    if (t >= p.vl[b].T) {
+      const size_t frame = (size_t)b * p.T + t;
+      if (tid < 128) {
+        if (p.mel_out) p.mel_out[frame * 128 + tid] = 0.f;
+        if (p.logmel_out) p.logmel_out[frame * 128 + tid] = 0.f;
+      }
+      return;
+    }
+  }
 
   // windowed, reflect-padded frame packed as z[n] = x[2n] + i x[2n+1]; 1024-point FFT (fft.cuh)
-  load_frame_packed(buf0, x, p.n, t, p.window, tid);
+  load_frame_packed(buf0, x, n, t, p.window, tid);
   __syncthreads();
   const float2* src = fft1024_forward(buf0, buf1, p.tw1024, tid);
   // src == buf1 now holds Z[0..1023]; buf0 is free and becomes the magnitude row

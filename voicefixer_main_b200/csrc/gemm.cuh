@@ -93,6 +93,13 @@ struct GemmEpilogue {
   int tma_out;           // bit 3: MAP_CONVT1D out_a through a 5-D map (see gemm_tc.cu).  MAP_PLAIN layers: bit 0 out_raw, bit 1 out_r, bit 2 out_a leave the staging tiles by TMA store
                          // (GemmTcParams::o_raw / o_r / o_a) instead of LDS + STG: half the LSU wavefronts of the store path
   int* err;
+  // Clips of different lengths in one batch (vf_restore_varlen): the per-image table of the call (kernels.cuh VarlenImage).
+  // vl_rows[img * vl_stride] = valid OUTPUT rows of image img (before out_row0); every output row at or past it is written
+  // as zeros (the value, not the old contents), so the next conv reads the same zero padding a clip of that length alone
+  // reads out of bounds.  vl_head_T[img * vl_stride] = frames the fused head writes.  Null: every row is valid.
+  const int* vl_rows;
+  const int* vl_head_T;
+  int vl_stride;
 };
 
 struct GemmProblem {
@@ -145,6 +152,8 @@ struct PairParams {
   uint32_t magic_t;              // gemm_tc_magic(tiles_per_img, ...)
   float slope_h, slope_out;
   int* err;
+  const int* vl_len;             // per-image clip length L_b = vl_len[img * vl_stride] (varlen batches, see GemmEpilogue), or
+  int vl_stride;                 // null: L.  Rows at or past L_b are zero in h and in both outputs
 };
 
 __host__ __device__ inline uint32_t fast_div_pair(uint32_t n, uint32_t d, uint32_t magic) {
@@ -190,8 +199,10 @@ __device__ __forceinline__ void epilogue_chunk(const GemmEpilogue& e, int img, i
     co0 = n_base - phase * e.cout;
   }
   size_t orow;
+  long lrow;               // output row inside the image
   bool pad = false;
   if (e.map == MAP_PLAIN) {
+    lrow = r;
     orow = (size_t)img * e.out_img_rows + e.out_row0 + r;
     if (e.Wp > 0) pad = (r % e.Wp) == e.Wp - 1;
   } else if (e.map == MAP_CONVT2D) {
@@ -199,13 +210,16 @@ __device__ __forceinline__ void epilogue_chunk(const GemmEpilogue& e, int img, i
     const int ph = phase >> 1, pw = phase & 1;
     const int col = 2 * w + pw;
     if (col >= e.ct_out_wp) return;          // both=True prune: column past the output pitch
-    orow = (size_t)img * e.out_img_rows + (size_t)(2 * h + ph) * e.ct_out_wp + col;
+    lrow = (long)(2 * h + ph) * e.ct_out_wp + col;
+    orow = (size_t)img * e.out_img_rows + lrow;
     pad = col == e.ct_out_wp - 1;
   } else {
     const long t = (long)r * e.ct_stride + phase - e.ct_pad;
     if (t < 0 || t >= e.out_rows_valid) return;
+    lrow = t;
     orow = (size_t)img * e.out_img_rows + e.out_row0 + t;
   }
+  if (e.vl_rows && lrow >= __ldg(e.vl_rows + (size_t)img * e.vl_stride)) pad = true;   // past this clip: zeros
   if (e.bias) {
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] += __ldg(e.bias + n_base + i);
@@ -266,6 +280,7 @@ __device__ __forceinline__ void epilogue_head(const GemmEpilogue& e, int img, in
   if (!e.head_w || r >= e.rows_in) return;
   const int t = r / e.Wp, f = r - t * e.Wp;
   if (t >= e.head_T) return;
+  if (e.vl_head_T && t >= __ldg(e.vl_head_T + (size_t)img * e.vl_stride)) return;
   const size_t idx = ((size_t)img * e.head_T + t) * e.Wp + f;
   const float y = (f < e.Wp - 1) ? head_acc + e.head_b : 0.f;
   e.head_out[idx] = e.head_in ? y + __ldg(e.head_in + idx) : y;

@@ -33,6 +33,14 @@ namespace {
 
 constexpr int kRowValid = 1, kRowPad = 2;
 
+// A clip's valid output rows (varlen batches, GemmEpilogue::vl_rows), read where it is used: as a volatile load it is not
+// hoisted or kept across the epilogue's tile loop (the two-CTA variants have no register to spare).
+__device__ __forceinline__ int ld_row_limit(const int* p) {
+  int v;
+  asm volatile("ld.global.nc.b32 %0, [%1];" : "=r"(v) : "l"(p));
+  return v;
+}
+
 struct RowInfo {        // published per epilogue thread for its own row, read by the lanes that store that row
   uint32_t orow;        // output row index (already includes image base / row0 / phase mapping)
   uint32_t flags;
@@ -430,10 +438,24 @@ __global__ void __launch_bounds__(64 + 32 * EPI_WARPS, MINB)
         if (row_ok) {
           orow = obase + lane;
           flags = kRowValid | ((Wp > 0 && (r % Wp) == Wp - 1) ? kRowPad : 0);
+          if (e.vl_rows && r >= __ldg(e.vl_rows + (size_t)img * e.vl_stride)) flags |= kRowPad;   // past this clip: zeros
         }
-      } else if (map == MAP_CONVT2D) {
-        cth = r / Wp;
-        ctw = r - cth * Wp;
+      } else {
+        if (map == MAP_CONVT2D) {
+          cth = r / Wp;
+          ctw = r - cth * Wp;
+        }
+        // varlen, 3-term kernels: bit 8 + p of flags = the output row of phase p lies past this clip, decided once per tile
+        // (the 1-term kernels test each chunk instead: whichever form costs the variant no spill)
+        if (THREE && e.vl_rows && row_ok) {
+          const int vlim = ld_row_limit(e.vl_rows + img * e.vl_stride);
+          const int nph = map == MAP_CONVT2D ? 4 : e.ct_stride;
+          for (int p = 0; p < nph; ++p) {
+            const long t = map == MAP_CONVT2D ? (long)(2 * cth + (p >> 1)) * e.ct_out_wp     // vlim: whole rows of pitch ct_out_wp
+                                              : (long)r * e.ct_stride + p - e.ct_pad;
+            if (t >= vlim) flags |= 1u << (8 + p);
+          }
+        }
       }
       // store this warp's staged 32 rows x 32 columns of fp16 (hi [+ lo]) row-major: 8 rows x 64 B per instruction
       auto store_rows_h = [&](const OutPlane& op, const int co0, const bool two, const CUtensorMap* tm) {
@@ -497,20 +519,25 @@ __global__ void __launch_bounds__(64 + 32 * EPI_WARPS, MINB)
         if (map != MAP_PLAIN) {           // transposed convs: the output row depends on the phase of this chunk
           const int phase = nb / cout;
           co0 = nb - phase * cout;
-          orow = 0; flags = 0;
+          const uint32_t keep = THREE ? flags & ~0xffu : 0u;
+          const uint32_t past = THREE && ((flags >> (8 + phase)) & 1u) ? (uint32_t)kRowPad : 0u;
+          orow = 0; flags = keep;
           if (row_ok) {
             if (map == MAP_CONVT2D) {
               const int ph = phase >> 1, pw = phase & 1;
               const int col = 2 * ctw + pw;
               if (col < e.ct_out_wp) {         // both=True pruning drops the column past the output pitch
-                orow = (uint32_t)((size_t)img * e.out_img_rows + (size_t)(2 * cth + ph) * e.ct_out_wp + col);
-                flags = kRowValid | (col == e.ct_out_wp - 1 ? kRowPad : 0);
+                const int lrow = (2 * cth + ph) * e.ct_out_wp + col;
+                orow = (uint32_t)((size_t)img * e.out_img_rows + lrow);
+                flags = keep | past | kRowValid | (col == e.ct_out_wp - 1 ? kRowPad : 0);
+                if (!THREE && e.vl_rows && lrow >= ld_row_limit(e.vl_rows + img * e.vl_stride)) flags |= kRowPad;
               }
             } else {
               const long t = (long)r * e.ct_stride + phase - e.ct_pad;
               if (t >= 0 && t < e.out_rows_valid) {
                 orow = (uint32_t)((size_t)img * e.out_img_rows + e.out_row0 + t);
-                flags = kRowValid;
+                flags = keep | past | kRowValid;
+                if (!THREE && e.vl_rows && t >= ld_row_limit(e.vl_rows + img * e.vl_stride)) flags |= kRowPad;
               }
             }
           }
@@ -608,7 +635,7 @@ __global__ void __launch_bounds__(64 + 32 * EPI_WARPS, MINB)
               add_planes(v[8 * i + 2 * k], v[8 * i + 2 * k + 1], reinterpret_cast<const uint32_t*>(ph)[k], reinterpret_cast<const uint32_t*>(pl)[k], resid_ar);
           }
         }
-        const bool pad = (flags & kRowPad) != 0;
+        const bool pad = (flags & kRowPad) != 0;      // pad column, or a row past its clip (varlen): zeros before any range check
         if (pad) {
 #pragma unroll
           for (int i = 0; i < 32; ++i) v[i] = 0.f;

@@ -6,6 +6,31 @@
 
 namespace vf {
 
+// Clips of different lengths in one batch (vf_restore_varlen).  A small kernel writes one record per clip at the start of
+// every call; every later kernel of the call reads its clip's lengths from it in device memory, so a captured launch chain
+// stays valid whatever the lengths are.  All rows at or past a clip's length in a plane a later conv reads are written as
+// zeros: what an earlier call with longer clips left in the slot never matters.
+constexpr int VF_VARLEN_MAX_CLIPS = 128;     // lengths travel by value in the setup kernel's parameter block
+struct VarlenImage {
+  int n;              // valid input samples
+  int T;              // frames, 1 + n / hop
+  int Tp;             // T padded to a multiple of 64 (the UNet's zero input rows, unet.py:75-77)
+  int unet_rows[7];   // valid rows of UNet level l: (Tp >> l) * Wp_l
+  int voc_len[9];     // vocoder lengths: [0] = Tv = T + T % 2 + tail base, [s + 1] = output length of up-sampling stage s
+  int L;              // vocoder output samples
+  int skip;           // centre-trim offset (L - n) / 2
+  int pad_[3];
+};
+constexpr int VARLEN_STRIDE = (int)(sizeof(VarlenImage) / sizeof(int));
+static_assert(sizeof(VarlenImage) % 16 == 0, "VarlenImage: keep records 16-byte aligned");
+struct VarlenSetupParams {
+  int batch, W0, hop, tail_base, num_stages;
+  int scales[8];
+  VarlenImage* out;    // [batch]
+  long long n[VF_VARLEN_MAX_CLIPS];
+};
+cudaError_t launch_varlen_setup(const VarlenSetupParams& p, cudaStream_t stream);
+
 struct FrontendParams {
   const float* wav;      // [batch, n]
   long n;
@@ -22,6 +47,8 @@ struct FrontendParams {
   float* sin_out;
   float* mel_out;        // [batch, T, 128] linear mel or null
   float* logmel_out;     // [batch, T, 128] log10(clip(mel, 1e-8)) or null
+  const VarlenImage* vl; // or null.  Set: n is the row stride of wav, clip b has vl[b].n samples and vl[b].T frames;
+                         // frames past them are written as zeros
 };
 cudaError_t launch_frontend(const FrontendParams& p, cudaStream_t stream);
 
@@ -47,6 +74,7 @@ struct UnetFirstParams {
   PlanePtr a2;           // [batch, Tp*Wp, 32] act(bn2(conv1(...))), pad column zero
   float* sc_raw;         // [batch, Tp*Wp, 32] fp32 shortcut(x), pad column zero
   int* err;
+  const VarlenImage* vl; // or null.  Set: T is the row stride of logmel; clip b uses vl[b].T / vl[b].Tp, rows past Tp_b are 0
 };
 cudaError_t launch_unet_first(const UnetFirstParams& p, cudaStream_t stream);
 
@@ -62,6 +90,8 @@ struct PoolParams {
   const float* a_shift;
   float slope;
   int* err;
+  const VarlenImage* vl; // or null.  Set: output rows at or past vl[b].unet_rows[vl_level] are written as zeros
+  int vl_level;          // UNet level of the output
 };
 cudaError_t launch_pool(const PoolParams& p, cudaStream_t stream);
 
@@ -79,19 +109,22 @@ struct VocCondParams {
   const float* band_sums;    // [batch][2] (target, estimate) low-band sums from launch_band_energy, or null:
                              // amp_to_original_f (tools/utils.py:50-55) scales the estimate by target/estimate
   PlanePtr out;          // [batch, Tv, 128]
+  const VarlenImage* vl; // or null.  Set: T is the row stride of mel; clip b: mel rows [0, T_b), the tail on [T_b, Tv_b), zeros after
 };
 cudaError_t launch_voc_condition(const VocCondParams& p, cudaStream_t stream);
 
 // amp_to_original_f, reduction half: per clip, sums over frames and mel bins [5, int(128*0.2)) of the noisy
 // linear mel (target) and of from_log(restored log-mel) (estimate).  sums must be zeroed before the launch.
 cudaError_t launch_band_energy(const float* mel_target_lin, const float* logmel_est, int batch, int T, float* sums,
-                               cudaStream_t stream);
+                               cudaStream_t stream, const VarlenImage* vl = nullptr);   // vl: T is the row stride, sums over T_b
 
 // amp_to_original_f as a stand-alone op: out = est * (low-band mean of target / low-band mean of est), linear mels [batch, T, 128].
 cudaError_t launch_amp_to_original(const float* est, const float* tgt, int batch, int T, float* out, cudaStream_t stream);
 
 // nn.ReflectionPad1d(3): rows [3, L+3) of each image are already written; fill 3 + 3 mirrored rows.
-cudaError_t launch_reflect_fill(PlanePtr planes, int batch, int L, int C, int pad, cudaStream_t stream);
+// vl (or null): L is the row pitch less 2 * pad; clip b reflects at its own length vl[b].voc_len[vl_stage].
+cudaError_t launch_reflect_fill(PlanePtr planes, int batch, int L, int C, int pad, cudaStream_t stream,
+                                const VarlenImage* vl = nullptr, int vl_stage = 0);
 
 // Tail: ReflectionPad(3) (pre-filled) + Conv1d(C -> 1, k7) + tanh, plus the per-clip peak |out|.
 struct VocTailParams {
@@ -102,6 +135,7 @@ struct VocTailParams {
   float bias;
   float* wav;            // [batch, L]
   unsigned int* peak_bits;   // [batch] max |out| as float bits (non-negative floats order like uints)
+  const VarlenImage* vl;     // or null.  Set: clip b has vl[b].L samples (peak over those only, zeros after them)
 };
 cudaError_t launch_voc_tail(const VocTailParams& p, cudaStream_t stream);
 
@@ -113,6 +147,7 @@ struct FinalizeParams {
   long L, n, skip;       // out[b, i] = wav[b, skip + i], i < n
   float* out;            // [batch, out_ld]
   long out_ld, out_off;
+  const VarlenImage* vl; // or null.  Set: clip b keeps vl[b].n samples from vl[b].skip; out[b, i] = 0 for vl[b].n <= i < n
 };
 cudaError_t launch_finalize(const FinalizeParams& p, cudaStream_t stream);
 cudaError_t launch_pcm16(const float* in, int16_t* out, size_t n, int saturate, cudaStream_t stream);

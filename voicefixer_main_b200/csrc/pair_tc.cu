@@ -224,7 +224,8 @@ __global__ void __launch_bounds__(PAIR_THREADS, 1) pair_tc_kernel(const __grid_c
       const int m0 = (tile - img * P.tiles_per_img) * PAIR_ROWS - 1;
       const int b = j & 1;
       const int t = m0 + jrow;
-      const bool in_clip = t >= 0 && t < P.L;
+      const int len = P.vl_len ? __ldg(P.vl_len + (size_t)img * P.vl_stride) : P.L;     // varlen batch: this clip's length
+      const bool in_clip = t >= 0 && t < len;
       if (!mbar_wait(acc1_full + b, (j >> 1) & 1, P.err, ERR_PIPE_EPILOGUE)) { ok = false; break; }
       tc_fence_after();
       if (!mbar_wait(h_free, (j & 1) ^ 1, P.err, ERR_PIPE_EPILOGUE)) { ok = false; break; }      // P2(j-1) has read H
@@ -317,6 +318,15 @@ __global__ void __launch_bounds__(PAIR_THREADS, 1) pair_tc_kernel(const __grid_c
           }
         }
         if (!AR) e2_bar_sync();                // the fp32 result overwrites the plane tiles other warps still read
+      }
+      if (P.vl_len) {                          // varlen batch: rows past this clip leave as zeros (x_new and the activated tile)
+        const int tile = blockIdx.x + j * gridDim.x;
+        const int img = (int)fast_div_pair((uint32_t)tile, (uint32_t)P.tiles_per_img, P.magic_t);
+        const int t = (tile - img * P.tiles_per_img) * PAIR_ROWS + xrow;
+        if (t >= __ldg(P.vl_len + (size_t)img * P.vl_stride)) {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = 0.f;
+        }
       }
       if (want_f && row_valid) {               // x_new in place: fp32 half tile `half`
         uint8_t* rp = xs + half * PAIR_X_TILE + (size_t)xrow * 128;

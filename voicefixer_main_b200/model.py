@@ -13,6 +13,7 @@ Same names, arguments and error behaviour as the objects eval_gsr_voicefixer.py:
     plus the batched fused entry points the reference lacks:
       .restore(wav[B,N]) -> wav[B,N]             one launch chain for stages A -> B -> C + normalise + trim
       .restore_host(pinned_in, pinned_out)
+      .restore_many([wav_i, ...]) -> [out_i, ...]  clips of any lengths, batched (Engine.restore_varlen)
 
 PyTorch is used only to own device memory and streams; every tensor handed back is written by a
 hand-written sm_100a kernel.  Tensors must be fp32 CUDA tensors on the model's device.
@@ -66,6 +67,16 @@ def melscale_fbanks(n_freqs=1025, f_min=0.0, f_max=22050.0, n_mels=128, sample_r
     down_slopes = (-1.0 * slopes[:, :-2]) / f_diff[:-1]
     up_slopes = slopes[:, 2:] / f_diff[1:]
     return torch.max(torch.zeros(1), torch.min(down_slopes, up_slopes))
+
+
+def group_sizes(n: int, max_batch: int):
+    """Sizes of the groups restore_many splits n sorted clips into: ceil(n / max_batch) groups, none above max_batch, sizes
+    differing by at most one (larger groups first)."""
+    if n <= 0:
+        return []
+    k = -(-n // max_batch)
+    q, r = divmod(n, k)
+    return [q + 1] * r + [q] * (k - r)
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -199,6 +210,28 @@ class Engine:
         flags = L.VF_RESTORE_UNIFY_ENERGY if unify_energy else 0
         with torch.cuda.device(self.device):
             self._ck(self.lib.vf_restore_ex(self.ctx, _ptr(wav), b, n, _ptr(out), flags, _stream()))
+        return out
+
+    def restore_varlen(self, wav: torch.Tensor, lengths, out: Optional[torch.Tensor] = None,
+                       unify_energy: bool = False) -> torch.Tensor:
+        """restore() over clips of different lengths: wav [B, n_max], row b holds lengths[b] valid samples (the rest is
+        never read).  Row b of the result is bit-identical to restore() of that clip alone; samples past lengths[b] are 0."""
+        wav = _check_in(wav, self.device, "wav")
+        if wav.dim() != 2:
+            raise ValueError(f"wav must be [B, n_max], got shape {tuple(wav.shape)}")
+        b, n = wav.shape
+        lens = [int(x) for x in lengths]
+        if len(lens) != b:
+            raise ValueError(f"restore_varlen: {len(lens)} lengths for a batch of {b}")
+        bad = [(i, x) for i, x in enumerate(lens) if not 1024 < x <= n]
+        if bad:
+            raise ValueError(f"restore_varlen: every length must satisfy 1024 < length <= n_max = {n}; "
+                             f"got {bad[:4]} (clip, length)")
+        out = torch.empty_like(wav) if out is None else out
+        flags = L.VF_RESTORE_UNIFY_ENERGY if unify_energy else 0
+        arr = (ctypes.c_int64 * b)(*lens)
+        with torch.cuda.device(self.device):
+            self._ck(self.lib.vf_restore_varlen(self.ctx, _ptr(wav), b, n, arr, _ptr(out), flags, _stream()))
         return out
 
     def mel(self, specgram: torch.Tensor) -> torch.Tensor:
@@ -611,6 +644,34 @@ class VoiceFixer(_EngineModel):
         if pip_kwargs:
             raise TypeError(f"restore(tensor): unexpected arguments {sorted(pip_kwargs)}")
         return self._engine().restore(wav, out, unify_energy=unify_energy)
+
+    def restore_many(self, wavs, unify_energy: bool = False, max_batch: int = 32) -> list:
+        """Restore a list of 1-D clips of any lengths (each more than 1024 samples) in batched calls; returns the restored
+        clips (1-D, on the model's device) in input order, each bit-identical to restore() of that clip alone.
+
+        The clips are sorted by length and split into ceil(len / max_batch) groups of near-equal size (so the last group
+        does not build a plan of an odd batch size); each group is padded to its longest clip and goes through ONE
+        restore_varlen call.  Sorting keeps the padded work small: neighbours in length share a group."""
+        if max_batch < 1:
+            raise ValueError("max_batch must be at least 1")
+        clips = [torch.as_tensor(w).reshape(-1) for w in wavs]
+        if not clips:
+            return []
+        eng = self._engine()
+        order = sorted(range(len(clips)), key=lambda i: clips[i].shape[0])
+        groups = group_sizes(len(clips), max_batch)
+        result = [None] * len(clips)
+        pos = 0
+        for g in groups:
+            idx = order[pos:pos + g]
+            pos += g
+            lens = [clips[i].shape[0] for i in idx]
+            batch = torch.nn.utils.rnn.pad_sequence([clips[i].to(device=eng.device, dtype=torch.float32) for i in idx],
+                                                    batch_first=True)
+            out = eng.restore_varlen(batch.contiguous(), lens, unify_energy=unify_energy)
+            for row, i in enumerate(idx):
+                result[i] = out[row, :lens[row]]
+        return result
 
     def restore_inmem(self, wav_10k, cuda=True, mode=0, your_vocoder_func=None):
         """The pip package's in-memory entry point: 44.1 kHz samples -> restored [1, N] numpy (handler.restore_inmem)."""
