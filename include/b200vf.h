@@ -23,6 +23,7 @@
  *                                 SSR_UNet / GSR_UNet inference (BASELINE config 3): models/ssr_unet.py:140-155 ->
  *                                 Generator.forward :51-54 -> unet_v2 UNetResComplex_100Mb.forward
  *                                 models/components/unet_v2.py:86-148 (magnitude net, input phase, ISTFT)
+ *   vf_ssr_restore_varlen         vf_ssr_restore over a batch of clips of different lengths (each row as if restored alone)
  *   vf_istft                      FDomainHelper.istft tools/pytorch/modules/fDomainHelper.py:30-32,127 (torchlibrosa ISTFT)
  *   vf_resample_poly              load_wav's rate conversion, tools/utils.py:46-48
  *   vf_lsd / vf_sispec            AudioMetrics.lsd / .sispec evaluation_proc/metrics.py:83-95 (handler's mel metrics,
@@ -156,6 +157,13 @@ VF_API int vf_ssr_forward(vf_ctx* ctx, const float* sp, const float* wav, int ba
 VF_API int vf_ssr_restore(vf_ctx* ctx, const float* wav, int batch, int64_t n_samples, float* wav_out, void* stream);
 VF_API int vf_ssr_restore_host(vf_ctx* ctx, const float* wav_host, int batch, int64_t n_samples, float* out_host,
                                void* stream);
+/* vf_ssr_restore over clips of different lengths, with the contract of vf_restore_varlen: wav [B, n_max] device, row b
+ * holds n_samples[b] valid samples (the rest is never read); n_samples is a HOST array, 1024 < n_samples[b] <= n_max,
+ * checked before anything is launched (VF_EINVAL).  wav_out [B, n_max]: row b is bit-identical to vf_ssr_restore of that
+ * clip alone; samples past n_samples[b] are 0.  Plans are cached per (batch, 64-frame bucket of the longest clip); batches
+ * above 128 clips (or above the plan budget) run as sub-batches. */
+VF_API int vf_ssr_restore_varlen(vf_ctx* ctx, const float* wav, int batch, int64_t n_max, const int64_t* n_samples,
+                                 float* wav_out, void* stream);
 /* The magnitude branch alone (unet_v2.py:99-132): sp [B,T,1025] -> out_mag [B,T,1025] (last bin 0, F.pad :128). */
 VF_API int vf_ssr_unet(vf_ctx* ctx, const float* sp, int batch, int frames, float* mag_out, void* stream);
 /* Intermediates of the last vf_ssr_* call of this shape: input magnitude and predicted magnitude [B,T,1025]. */
@@ -214,7 +222,7 @@ VF_API int vf_check_errors(vf_ctx* ctx, void* stream);
  * "host_pipeline" (default 1, see vf_restore_host),
  * "validate_simt" (1: run every GEMM on the SIMT validation kernel instead of tcgen05 - tests only). */
 VF_API int vf_set_option(vf_ctx* ctx, const char* key, int value);
-/* Plans are cached per (path, batch, frames) - frames rounded up to 64 for vf_restore_varlen; the cache is bounded (see "plan_cache_mb").  A batch whose plan would not fit
+/* Plans are cached per (path, batch, frames) - frames rounded up to 64 for vf_restore_varlen and vf_ssr_restore_varlen; the cache is bounded (see "plan_cache_mb").  A batch whose plan would not fit
  * the budget is processed in sub-batches through a smaller plan (same results: rows are independent); the *_stages accessors
  * then only see the last sub-batch. */
 VF_API int vf_plan_cache_info(vf_ctx* ctx, int* n_plans, size_t* bytes, size_t* budget, int64_t* evicted);

@@ -20,7 +20,7 @@ EXPORTS = [
     "vf_enable_stage_timing", "vf_stage_times", "vf_selftest_gemm", "vf_enable_op_timing", "vf_op_count", "vf_op_info",
     "vf_restore_ex", "vf_ssr_forward", "vf_ssr_restore", "vf_ssr_restore_host", "vf_ssr_unet", "vf_ssr_stages", "vf_istft",
     "vf_mel", "vf_finalize", "vf_plan_cache_info", "vf_resample_poly", "vf_lsd", "vf_sispec", "vf_to_pcm16_ex", "vf_amp_to_original_f",
-    "vf_restore_varlen",
+    "vf_restore_varlen", "vf_ssr_restore_varlen",
 ]
 VF_RESTORE_UNIFY_ENERGY = 1
 
@@ -98,6 +98,7 @@ def load_library():
     lib.vf_ssr_forward.argtypes = [P, P, P, c_int, c_int64, P, P]
     lib.vf_ssr_restore.argtypes = [P, P, c_int, c_int64, P, P]
     lib.vf_ssr_restore_host.argtypes = [P, P, c_int, c_int64, P, P]
+    lib.vf_ssr_restore_varlen.argtypes = [P, P, c_int, c_int64, POINTER(c_int64), P, P]
     lib.vf_ssr_unet.argtypes = [P, P, c_int, c_int, P, P]
     lib.vf_ssr_stages.argtypes = [P, c_int, c_int64, P, P, P]
     lib.vf_istft.argtypes = [P, P, P, c_int, c_int, c_int64, P, P]

@@ -116,9 +116,10 @@ struct UnetW {
   float head_b = 0;
 };
 
-// PLAN_GSR_VARLEN: the GSR chain over clips of different lengths (vf_restore_varlen), keyed by the 64-frame bucket of the
-// longest clip; its kernels take the per-clip lengths from the plan's VarlenImage table
-enum PlanKind { PLAN_GSR = 0, PLAN_SSR = 1, PLAN_GSR_VARLEN = 2 };
+// PLAN_GSR_VARLEN / PLAN_SSR_VARLEN: the GSR / SSR chain over clips of different lengths (vf_restore_varlen /
+// vf_ssr_restore_varlen), keyed by the 64-frame bucket of the longest clip; its kernels take the per-clip lengths from the
+// plan's VarlenImage table
+enum PlanKind { PLAN_GSR = 0, PLAN_SSR = 1, PLAN_GSR_VARLEN = 2, PLAN_SSR_VARLEN = 3 };
 
 struct Plan {
   int kind = PLAN_GSR;
@@ -142,7 +143,7 @@ struct Plan {
   float* d_logmel_out = nullptr; // [B, T, 128]
   float* d_voc_wav = nullptr;    // [B, L]
   float* d_band = nullptr;       // [B][2] low-band energy sums (unify_energy)
-  VarlenImage* d_vl = nullptr;   // [B] per-clip lengths of the current call (PLAN_GSR_VARLEN only)
+  VarlenImage* d_vl = nullptr;   // [B] per-clip lengths of the current call (PLAN_GSR_VARLEN / PLAN_SSR_VARLEN only)
   unsigned int* d_peak = nullptr;
   long L = 0;
   // SSR plans (unet_v2 + ISTFT)
@@ -1452,7 +1453,7 @@ int get_plan(vf_ctx* ctx, int kind, int batch, int frames, Plan** out) {
   if (!ctx->loaded) return fail(ctx, VF_ESTATE, "weights not loaded");
   if ((kind == PLAN_GSR || kind == PLAN_GSR_VARLEN) && !(ctx->gsr.loaded && ctx->voc_loaded))
     return fail(ctx, VF_ESTATE, "this entry point needs the analysis module (generator.analysis_module.*) and the vocoder (vocoder.*) weights");
-  if (kind == PLAN_SSR && !ctx->ssr.loaded)
+  if ((kind == PLAN_SSR || kind == PLAN_SSR_VARLEN) && !ctx->ssr.loaded)
     return fail(ctx, VF_ESTATE, "this entry point needs the unet_v2 weights (generator.unet.*)");
   // make room first: a failed cudaMalloc half way through a plan is slower to recover from than an early eviction
   {
@@ -1482,7 +1483,9 @@ int get_plan(vf_ctx* ctx, int kind, int batch, int frames, Plan** out) {
     if (!rc) rc = build_unet(ctx, b, plan.get(), ctx->gsr, g);
     if (!rc) rc = build_vocoder(ctx, b, plan.get());
   } else {
-    rc = build_ssr(ctx, b, plan.get());
+    if (kind == PLAN_SSR_VARLEN) plan->d_vl = b.alloc<VarlenImage>(batch);      // before build_unet: its ops point into it
+    rc = b.rc;
+    if (!rc) rc = build_ssr(ctx, b, plan.get());
   }
   if (rc == VF_ECUDA && !ctx->plans.empty()) {
     // out of memory with other plans cached: drop them all and retry once
@@ -1691,7 +1694,8 @@ int choose_sub_batch(vf_ctx* ctx, int kind, int batch, int frames) {
     if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) ctx->plan_budget = std::max<size_t>((free_b + ctx->plan_bytes) / 2, (size_t)1 << 30);
   }
   const double tp = (frames + 63) / 64 * 64;
-  double per_frame = kind == PLAN_SSR ? 2.4e6 : 1.7e6;      // bytes per clip and padded frame (measured 2.19e6 / 1.52e6) + margin
+  const bool ssr = kind == PLAN_SSR || kind == PLAN_SSR_VARLEN;
+  double per_frame = ssr ? 2.4e6 : 1.7e6;      // bytes per clip and padded frame (measured 2.19e6 / 1.52e6) + margin
   for (auto& kv : ctx->plans)
     if (std::get<0>(kv.first) == kind) {
       per_frame = 1.05 * (double)kv.second->bytes / ((double)kv.second->batch * ((kv.second->T + 63) / 64 * 64));
@@ -1982,7 +1986,10 @@ VF_API int vf_restore_host(vf_ctx* ctx, const float* wav_host, int batch, int64_
 }
 
 // ---------------------------------------------------------------------------------------------- SSR / GSR-UNet path
-static int ssr_impl(vf_ctx* ctx, Plan* plan, const float* sp, const float* wav, int batch, int64_t n, float* wav_out, cudaStream_t st) {
+// lens == null: every clip has n samples.  Else (a PLAN_SSR_VARLEN plan, sp null) clip b has lens[b] samples
+// (1024 < lens[b] <= n, checked by the caller), n is the row stride of wav and wav_out, and plan->T the 64-frame bucket.
+static int ssr_impl(vf_ctx* ctx, Plan* plan, const float* sp, const float* wav, int batch, int64_t n, float* wav_out, cudaStream_t st,
+                    const int64_t* lens = nullptr) {
   const int frames = plan->T;
   if (ctx->op_timing) ctx->prof.clear();
   int rc = plan_enter(ctx, plan, st);
@@ -1993,8 +2000,17 @@ static int ssr_impl(vf_ctx* ctx, Plan* plan, const float* sp, const float* wav, 
       if (!e) CK(cudaEventCreate(&e));
     CK(cudaEventRecord(ctx->ev[0], st));
   }
+  if (lens) {     // the per-clip table of this call (unet_v2 geometry, W0 = 1024): a plain launch ahead of everything else
+    VarlenSetupParams vp;
+    memset(&vp, 0, sizeof vp);
+    vp.batch = batch; vp.W0 = 1024; vp.hop = ctx->cfg.hop;      // the vocoder fields stay 0: no vocoder on this path
+    vp.out = plan->d_vl;
+    for (int b = 0; b < batch; ++b) vp.n[b] = (long long)lens[b];
+    CK(launch_varlen_setup(vp, st));
+    ctx->launches++;
+  }
   if (!sp) {     // SSR_UNet.pre (ssr_unet.py:140-143): the magnitude of the input itself
-    rc = run_frontend(ctx, wav, batch, (long)n, nullptr, nullptr, plan->d_sp, nullptr, nullptr, st);
+    rc = run_frontend(ctx, wav, batch, (long)n, nullptr, nullptr, plan->d_sp, nullptr, nullptr, st, plan->d_vl, frames);
     if (rc) return rc;
   }
   if (tm) CK(cudaEventRecord(ctx->ev[1], st));
@@ -2007,11 +2023,12 @@ static int ssr_impl(vf_ctx* ctx, Plan* plan, const float* sp, const float* wav, 
   memset(&fp, 0, sizeof fp);
   fp.mag = plan->d_mag; fp.wav = wav; fp.n = (long)n; fp.batch = batch; fp.T = frames;
   fp.window = ctx->d_window; fp.tw1024 = ctx->d_tw1024; fp.tw2048 = ctx->d_tw2048; fp.frames = plan->d_frames;
+  fp.vl = plan->d_vl;
   CK(launch_istft_frames(fp, st));
   IstftOlaParams op;
   memset(&op, 0, sizeof op);
   op.frames = plan->d_frames; op.batch = batch; op.T = frames; op.length = (long)n; op.window = ctx->d_window;
-  op.out = wav_out; op.out_ld = (long)n;
+  op.out = wav_out; op.out_ld = (long)n; op.vl = plan->d_vl;
   CK(launch_istft_ola(op, st));
   ctx->launches += 2;
   if (tm) { CK(cudaEventRecord(ctx->ev[3], st)); CK(cudaEventRecord(ctx->ev[4], st)); ctx->ev_valid = true; }
@@ -2038,6 +2055,35 @@ VF_API int vf_ssr_forward(vf_ctx* ctx, const float* sp, const float* wav, int ba
 
 VF_API int vf_ssr_restore(vf_ctx* ctx, const float* wav, int batch, int64_t n, float* wav_out, void* stream) {
   return vf_ssr_forward(ctx, nullptr, wav, batch, n, wav_out, stream);
+}
+
+VF_API int vf_ssr_restore_varlen(vf_ctx* ctx, const float* wav, int batch, int64_t n_max, const int64_t* n_samples,
+                                 float* wav_out, void* stream) {
+  int rc = check_ready(ctx);
+  if (rc) return rc;
+  if (!wav || !wav_out || !n_samples || batch <= 0) return fail(ctx, VF_EINVAL, "vf_ssr_restore_varlen: bad arguments");
+  if (n_max > (int64_t)INT32_MAX / 2) return fail(ctx, VF_EINVAL, "vf_ssr_restore_varlen: n_max %ld too large", (long)n_max);
+  // every length is checked before anything is launched
+  int64_t longest = 0;
+  for (int b = 0; b < batch; ++b) {
+    if (n_samples[b] <= 1024 || n_samples[b] > n_max)
+      return fail(ctx, VF_EINVAL, "vf_ssr_restore_varlen: clip %d has %ld samples; need 1024 < n <= n_max = %ld (reflect "
+                  "padding needs more than n_fft/2 samples)", b, (long)n_samples[b], (long)n_max);
+    longest = std::max(longest, n_samples[b]);
+  }
+  // one plan per (batch, 64-frame bucket of the longest clip), as for vf_restore_varlen
+  const int bucket = round_up(frames_of(ctx, (long)longest), 64);
+  const int cb = std::min(choose_sub_batch(ctx, PLAN_SSR_VARLEN, batch, bucket), VF_VARLEN_MAX_CLIPS);
+  for (int off = 0; off < batch; off += cb) {
+    const int b = std::min(cb, batch - off);
+    Plan* plan;
+    rc = get_plan(ctx, PLAN_SSR_VARLEN, b, bucket, &plan);
+    if (rc) return rc;
+    rc = ssr_impl(ctx, plan, nullptr, wav + (size_t)off * n_max, b, n_max, wav_out + (size_t)off * n_max, (cudaStream_t)stream,
+                  n_samples + off);
+    if (rc) return rc;
+  }
+  return VF_OK;
 }
 
 VF_API int vf_ssr_restore_host(vf_ctx* ctx, const float* wav_host, int batch, int64_t n, float* out_host, void* stream) {

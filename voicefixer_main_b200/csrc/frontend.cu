@@ -30,6 +30,11 @@ __global__ void __launch_bounds__(256) frontend_kernel(FrontendParams p) {
         if (p.mel_out) p.mel_out[frame * 128 + tid] = 0.f;
         if (p.logmel_out) p.logmel_out[frame * 128 + tid] = 0.f;
       }
+      if (p.sp_out)
+        for (int k = tid; k <= 1024; k += 256) {
+          p.sp_out[frame * 1025 + k] = 0.f;
+          if (p.cos_out) { p.cos_out[frame * 1025 + k] = 0.f; p.sin_out[frame * 1025 + k] = 0.f; }
+        }
       return;
     }
   }

@@ -22,8 +22,10 @@ __global__ void __launch_bounds__(256) istft_frames_kernel(IstftFramesParams p) 
   __shared__ float2 Y[1025];
   const int t = blockIdx.x, b = blockIdx.y, tid = threadIdx.x;
   const size_t frame = (size_t)b * p.T + t;
+  if (p.vl && t >= p.vl[b].T) return;       // past a varlen clip's frames: nothing to compute (uniform per CTA)
   if (p.mag) {
-    load_frame_packed(buf0, p.wav + (size_t)b * p.n, p.n, t, p.window, tid);
+    const long n = p.vl ? (long)p.vl[b].n : p.n;     // a varlen clip reflects at its own end
+    load_frame_packed(buf0, p.wav + (size_t)b * p.n, n, t, p.window, tid);
     __syncthreads();
     const float2* Z = fft1024_forward(buf0, buf1, p.tw1024, tid);
     for (int k = tid; k <= 1024; k += 256) {
@@ -64,16 +66,23 @@ cudaError_t launch_istft_frames(const IstftFramesParams& p, cudaStream_t stream)
   return cudaGetLastError();
 }
 
-// y[p] = sum_t frames[t][p - 441 t] / clamp(sum_t win^2[p - 441 t], 1e-11), p = i + 1024; ascending t (deterministic)
+// y[p] = sum_t frames[t][p - 441 t] / clamp(sum_t win^2[p - 441 t], 1e-11), p = i + 1024; ascending t (deterministic).
+// A varlen clip ends its sum at its own last frame T_b - 1: frame T_b starts at 441 T_b < 1024 + n_b, so it would
+// overlap the clip's last samples, and its window would enter the denominator even with a zero numerator.
 __global__ void __launch_bounds__(256) istft_ola_kernel(IstftOlaParams p) {
   const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
   const int b = blockIdx.y;
   if (i >= p.length) return;
+  long T = p.T;
+  if (p.vl) {
+    if (i >= p.vl[b].n) { p.out[(size_t)b * p.out_ld + i] = 0.f; return; }
+    T = p.vl[b].T;
+  }
   const long pos = i + 1024;
   long t_lo = (pos - 2047 + 440) / 441;       // ceil((pos - 2047) / 441), pos >= 1024 so the numerator may be negative
   if (pos - 2047 <= 0) t_lo = 0;
   long t_hi = pos / 441;
-  if (t_hi > p.T - 1) t_hi = p.T - 1;
+  if (t_hi > T - 1) t_hi = T - 1;
   float acc = 0.f, ws = 0.f;
   for (long t = t_lo; t <= t_hi; ++t) {
     const int off = (int)(pos - 441 * t);

@@ -6,7 +6,7 @@
 
 namespace vf {
 
-// Clips of different lengths in one batch (vf_restore_varlen).  A small kernel writes one record per clip at the start of
+// Clips of different lengths in one batch (vf_restore_varlen, vf_ssr_restore_varlen).  A small kernel writes one record per clip at the start of
 // every call; every later kernel of the call reads its clip's lengths from it in device memory, so a captured launch chain
 // stays valid whatever the lengths are.  All rows at or past a clip's length in a plane a later conv reads are written as
 // zeros: what an earlier call with longer clips left in the slot never matters.
@@ -48,7 +48,7 @@ struct FrontendParams {
   float* mel_out;        // [batch, T, 128] linear mel or null
   float* logmel_out;     // [batch, T, 128] log10(clip(mel, 1e-8)) or null
   const VarlenImage* vl; // or null.  Set: n is the row stride of wav, clip b has vl[b].n samples and vl[b].T frames;
-                         // frames past them are written as zeros
+                         // frames past them are written as zeros in every output that is set (all 1025 bins of sp / cos / sin)
 };
 cudaError_t launch_frontend(const FrontendParams& p, cudaStream_t stream);
 
@@ -185,6 +185,8 @@ struct IstftFramesParams {
   const float2* tw1024;
   const float2* tw2048;
   float* frames;         // [batch, T, 2048]
+  const VarlenImage* vl; // or null.  Set: n is the row stride of wav and T of mag / frames; clip b reflects at vl[b].n and
+                         // only its frames t < vl[b].T are computed (later frames are left as they are: no kernel reads them)
 };
 cudaError_t launch_istft_frames(const IstftFramesParams& p, cudaStream_t stream);
 struct IstftOlaParams {
@@ -194,6 +196,9 @@ struct IstftOlaParams {
   const float* window;
   float* out;            // [batch, out_ld]
   long out_ld;
+  const VarlenImage* vl; // or null.  Set: T is the row stride of frames, length the output samples per row; clip b sums its
+                         // frames t < vl[b].T only (numerator AND window-square sum, as if restored alone), writes vl[b].n
+                         // samples and exact zeros on [vl[b].n, length)
 };
 cudaError_t launch_istft_ola(const IstftOlaParams& p, cudaStream_t stream);
 

@@ -15,7 +15,7 @@ import wave
 import numpy as np
 import torch
 
-from .model import VoiceFixer, default_hparams
+from .model import SSR_UNet, VoiceFixer, default_hparams
 
 model = None
 hp = None
@@ -121,11 +121,16 @@ def handler(input, output, target, ckpt, device, needrefresh=False, meta={}):
     return metrics
 
 
-def restore_files(mdl: VoiceFixer, inputs, outputs, meta={}, max_batch=32):
+def restore_files(mdl, inputs, outputs, meta={}, max_batch=32):
     """handler() over many files at once: each output file is byte-identical to handler(input, output, None, ...) with the
     same meta ("unify_energy", "saturate"), but the 60 s segments of ALL files are pooled into batched calls
     (VoiceFixer.restore_many: sorted by length, groups of at most `max_batch`).  Files are read like handler() reads them
-    (load_wav, any sample rate through the GPU resampler).  No target metrics: use handler() for those."""
+    (load_wav, any sample rate through the GPU resampler).  No target metrics: use handler() for those.
+
+    `mdl` may also be an SSR_UNet / GSR_UNet.  Each file then gets the bytes the GSR-UNet handler (eval_gsr_unet.py:37-75)
+    writes with this model: 60 s segments, each restored (SSR_UNet.restore_many) and peak-normalised on its own when
+    max|x| > 1, no trim (the ISTFT returns the input length), concatenated, then save_wave's int16 cast.
+    meta["saturate"] is honoured; meta["unify_energy"] is ignored, as that handler never reads meta."""
     inputs, outputs = list(inputs), list(outputs)
     if len(inputs) != len(outputs):
         raise ValueError(f"restore_files: {len(inputs)} inputs but {len(outputs)} outputs")
@@ -136,7 +141,12 @@ def restore_files(mdl: VoiceFixer, inputs, outputs, meta={}, max_batch=32):
         for seg in split_segments(wav.shape[0]):
             segs.append(torch.from_numpy(np.ascontiguousarray(wav[seg])))
             owner.append(k)
-    res = mdl.restore_many(segs, unify_energy=bool(meta.get("unify_energy", False)), max_batch=max_batch)
+    if isinstance(mdl, SSR_UNet):
+        res = mdl.restore_many(segs, max_batch=max_batch)
+        # eval_gsr_unet.py:66-67: the segment divided by its peak when that exceeds 1 (trim_center :70 keeps n samples)
+        res = [eng.finalize(out[None], out.shape[0])[0] for out in res]
+    else:
+        res = mdl.restore_many(segs, unify_energy=bool(meta.get("unify_energy", False)), max_batch=max_batch)
     pieces = [[] for _ in inputs]
     for k, out in zip(owner, res):
         pieces[k].append(out)

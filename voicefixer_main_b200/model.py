@@ -14,6 +14,8 @@ Same names, arguments and error behaviour as the objects eval_gsr_voicefixer.py:
       .restore(wav[B,N]) -> wav[B,N]             one launch chain for stages A -> B -> C + normalise + trim
       .restore_host(pinned_in, pinned_out)
       .restore_many([wav_i, ...]) -> [out_i, ...]  clips of any lengths, batched (Engine.restore_varlen)
+    SSR_UNet / GSR_UNet (models/ssr_unet.py, gsr_unet.py): .pre, model(sp, wav)['wav'], .restore(wav[B,N]) and
+      .restore_many([wav_i, ...])             clips of any lengths, batched (Engine.ssr_restore_varlen)
 
 PyTorch is used only to own device memory and streams; every tensor handed back is written by a
 hand-written sm_100a kernel.  Tensors must be fp32 CUDA tensors on the model's device.
@@ -77,6 +79,32 @@ def group_sizes(n: int, max_batch: int):
     k = -(-n // max_batch)
     q, r = divmod(n, k)
     return [q + 1] * r + [q] * (k - r)
+
+
+def restore_grouped(mdl, wavs, max_batch: int, run) -> list:
+    """The batching of the restore_many methods: sort the 1-D clips by length, split them into group_sizes groups, pad
+    each group to its longest clip ([g, n_max] on the model's device) and restore it with ONE `run(engine, batch,
+    lengths)` call, which returns [g, n_max]; the clips come back (1-D views of those rows) in input order."""
+    if max_batch < 1:
+        raise ValueError("max_batch must be at least 1")
+    clips = [torch.as_tensor(w).reshape(-1) for w in wavs]
+    if not clips:
+        return []
+    eng = mdl._engine()
+    order = sorted(range(len(clips)), key=lambda i: clips[i].shape[0])
+    groups = group_sizes(len(clips), max_batch)
+    result = [None] * len(clips)
+    pos = 0
+    for g in groups:
+        idx = order[pos:pos + g]
+        pos += g
+        lens = [clips[i].shape[0] for i in idx]
+        batch = torch.nn.utils.rnn.pad_sequence([clips[i].to(device=eng.device, dtype=torch.float32) for i in idx],
+                                                batch_first=True)
+        out = run(eng, batch.contiguous(), lens)
+        for row, i in enumerate(idx):
+            result[i] = out[row, :lens[row]]
+    return result
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -216,23 +244,29 @@ class Engine:
                        unify_energy: bool = False) -> torch.Tensor:
         """restore() over clips of different lengths: wav [B, n_max], row b holds lengths[b] valid samples (the rest is
         never read).  Row b of the result is bit-identical to restore() of that clip alone; samples past lengths[b] are 0."""
-        wav = _check_in(wav, self.device, "wav")
-        if wav.dim() != 2:
-            raise ValueError(f"wav must be [B, n_max], got shape {tuple(wav.shape)}")
+        wav, lens = self._varlen_args(wav, lengths, "restore_varlen")
         b, n = wav.shape
-        lens = [int(x) for x in lengths]
-        if len(lens) != b:
-            raise ValueError(f"restore_varlen: {len(lens)} lengths for a batch of {b}")
-        bad = [(i, x) for i, x in enumerate(lens) if not 1024 < x <= n]
-        if bad:
-            raise ValueError(f"restore_varlen: every length must satisfy 1024 < length <= n_max = {n}; "
-                             f"got {bad[:4]} (clip, length)")
         out = torch.empty_like(wav) if out is None else out
         flags = L.VF_RESTORE_UNIFY_ENERGY if unify_energy else 0
         arr = (ctypes.c_int64 * b)(*lens)
         with torch.cuda.device(self.device):
             self._ck(self.lib.vf_restore_varlen(self.ctx, _ptr(wav), b, n, arr, _ptr(out), flags, _stream()))
         return out
+
+    def _varlen_args(self, wav: torch.Tensor, lengths, what: str):
+        """The host-side checks of the varlen entry points: (wav, lengths as ints), or ValueError before any launch."""
+        wav = _check_in(wav, self.device, "wav")
+        if wav.dim() != 2:
+            raise ValueError(f"wav must be [B, n_max], got shape {tuple(wav.shape)}")
+        b, n = wav.shape
+        lens = [int(x) for x in lengths]
+        if len(lens) != b:
+            raise ValueError(f"{what}: {len(lens)} lengths for a batch of {b}")
+        bad = [(i, x) for i, x in enumerate(lens) if not 1024 < x <= n]
+        if bad:
+            raise ValueError(f"{what}: every length must satisfy 1024 < length <= n_max = {n}; "
+                             f"got {bad[:4]} (clip, length)")
+        return wav, lens
 
     def mel(self, specgram: torch.Tensor) -> torch.Tensor:
         """MelScale.forward: specgram [..., 1025, time] (any strides) -> [..., 128, time]."""
@@ -278,6 +312,18 @@ class Engine:
         out = torch.empty_like(wav) if out is None else out
         with torch.cuda.device(self.device):
             self._ck(self.lib.vf_ssr_forward(self.ctx, _ptr(sp), _ptr(wav), b, n, _ptr(out), _stream()))
+        return out
+
+    def ssr_restore_varlen(self, wav: torch.Tensor, lengths, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """ssr_forward(None, .) over clips of different lengths: wav [B, n_max], row b holds lengths[b] valid samples (the
+        rest is never read).  Row b of the result is bit-identical to SSR_UNet.restore of that clip alone; samples past
+        lengths[b] are 0."""
+        wav, lens = self._varlen_args(wav, lengths, "ssr_restore_varlen")
+        b, n = wav.shape
+        out = torch.empty_like(wav) if out is None else out
+        arr = (ctypes.c_int64 * b)(*lens)
+        with torch.cuda.device(self.device):
+            self._ck(self.lib.vf_ssr_restore_varlen(self.ctx, _ptr(wav), b, n, arr, _ptr(out), _stream()))
         return out
 
     def ssr_restore_host(self, wav_host: torch.Tensor, out_host: torch.Tensor):
@@ -652,26 +698,8 @@ class VoiceFixer(_EngineModel):
         The clips are sorted by length and split into ceil(len / max_batch) groups of near-equal size (so the last group
         does not build a plan of an odd batch size); each group is padded to its longest clip and goes through ONE
         restore_varlen call.  Sorting keeps the padded work small: neighbours in length share a group."""
-        if max_batch < 1:
-            raise ValueError("max_batch must be at least 1")
-        clips = [torch.as_tensor(w).reshape(-1) for w in wavs]
-        if not clips:
-            return []
-        eng = self._engine()
-        order = sorted(range(len(clips)), key=lambda i: clips[i].shape[0])
-        groups = group_sizes(len(clips), max_batch)
-        result = [None] * len(clips)
-        pos = 0
-        for g in groups:
-            idx = order[pos:pos + g]
-            pos += g
-            lens = [clips[i].shape[0] for i in idx]
-            batch = torch.nn.utils.rnn.pad_sequence([clips[i].to(device=eng.device, dtype=torch.float32) for i in idx],
-                                                    batch_first=True)
-            out = eng.restore_varlen(batch.contiguous(), lens, unify_energy=unify_energy)
-            for row, i in enumerate(idx):
-                result[i] = out[row, :lens[row]]
-        return result
+        return restore_grouped(self, wavs, max_batch,
+                               lambda eng, batch, lens: eng.restore_varlen(batch, lens, unify_energy=unify_energy))
 
     def restore_inmem(self, wav_10k, cuda=True, mode=0, your_vocoder_func=None):
         """The pip package's in-memory entry point: 44.1 kHz samples -> restored [1, N] numpy (handler.restore_inmem)."""
@@ -728,6 +756,13 @@ class SSR_UNet(_EngineModel):
     def restore(self, wav: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """pre + forward fused: wav [B,N] -> denoised [B,N] (the magnitude never leaves the device plan)."""
         return self._engine().ssr_forward(None, wav, out)
+
+    def restore_many(self, wavs, max_batch: int = 32) -> list:
+        """Restore a list of 1-D clips of any lengths (each more than 1024 samples) in batched calls; returns the restored
+        clips (1-D, on the model's device) in input order, each bit-identical to restore() of that clip alone.  Grouping
+        as VoiceFixer.restore_many (sorted by length, near-equal groups of at most `max_batch`, one ssr_restore_varlen
+        call per group).  Like restore(), no peak normalisation is applied."""
+        return restore_grouped(self, wavs, max_batch, lambda eng, batch, lens: eng.ssr_restore_varlen(batch, lens))
 
     def restore_host(self, wav_host: torch.Tensor, out_host: torch.Tensor):
         self._engine().ssr_restore_host(wav_host, out_host)
